@@ -2,6 +2,7 @@
 """bench.py -- DESC solve throughput on B200 (metric of BASELINE.json), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg4|cfg2|cfg3|cfg3sc|cfg5]
+                    [--dump-outputs DIR]
 
 A "step" is one complete DESC_init-equivalent solve (DESC.m:14-263 + GCW.m) of the workload:
 CSR incidence build + cycle inconsistencies + PGD (iterations actually run) + GCW recovery.
@@ -408,15 +409,16 @@ def run_gpu(args, wl):
     kw = dict(device=local, stream=stream.cuda_stream, rank=rank, world=world, nccl_id=nccl_id)
     state = {}
 
-    def step_resident():
+    def step_resident(fetch=False):
         s = desc_b200.Solver(Ind_d, R_d, n=n, **kw)
         try:
             info = s.build_incidence(n_sample=wl["n_sample"], seed=1)
             s.cycle_inconsistency()
-            _, _, iters_run = s.pgd(wl["iters"], rule, want_S=False, want_hist=False)
-            if wl.get("gcw", True):
-                s.gcw(want_R=False)
+            S_vec, _, iters_run = s.pgd(wl["iters"], rule, want_S=fetch, want_hist=False)
+            R_est = s.gcw(want_R=fetch) if wl.get("gcw", True) else None
             state.update(info=info, iters_run=iters_run, timings=s.timings())
+            if fetch:
+                state.update(S_vec=S_vec, R_est=R_est)
         finally:
             s.close()
 
@@ -434,16 +436,16 @@ def run_gpu(args, wl):
         finally:
             s.close()
 
-    def timed(fn, steps):
+    def timed(fn, steps, **last_kw):
         import gc
         gc.collect()
         gc.disable()            # no collector pauses of the host inside the timed region
         try:
-            return _timed(fn, steps)
+            return _timed(fn, steps, last_kw)
         finally:
             gc.enable()
 
-    def _timed(fn, steps):
+    def _timed(fn, steps, last_kw):
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize(dev)
@@ -451,9 +453,9 @@ def run_gpu(args, wl):
         ev0.record(stream)
         launches = 0
         trace = os.environ.get("DESC_BENCH_TRACE") == "1"   # diagnostics: host wall time of every step (adds a sync)
-        for _ in range(steps):
+        for i in range(steps):
             t0 = time.perf_counter()
-            fn()
+            fn(**(last_kw if i == steps - 1 else {}))
             if trace:
                 torch.cuda.synchronize(dev)
                 sys.stderr.write("step %s: %.1f ms\n" % (fn.__name__, 1e3 * (time.perf_counter() - t0)))
@@ -472,8 +474,10 @@ def run_gpu(args, wl):
     sampler = ClockSampler(local) if rank == 0 and os.environ.get("DESC_BENCH_NO_CLOCKS") != "1" else None
     for _ in range(args.warmup):
         step_resident()
-    ms_total, launches = timed(step_resident, args.steps)
+    ms_total, launches = timed(step_resident, args.steps, fetch=args.dump_outputs is not None)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, S_vec=state["S_vec"], R_est=state["R_est"])
     ms_step = ms_total / args.steps
     info, iters_run, tm = state["info"], state["iters_run"], state["timings"]
     evals = info["m_cycle"] * iters_run
@@ -505,8 +509,8 @@ def run_gpu(args, wl):
             side = {"error": "%s: %s" % (type(e).__name__, e)}
 
     step_e2e()
-    ms_e2e_total, _ = timed(step_e2e, max(1, min(args.steps, 3)))
-    ms_e2e = ms_e2e_total / max(1, min(args.steps, 3))
+    ms_e2e_total, _ = timed(step_e2e, args.steps)
+    ms_e2e = ms_e2e_total / args.steps
     e2e = {"value": evals / (ms_e2e * 1e-3), "unit": UNIT, "h2d_bytes_per_step": (2 * m + 9 * m) * 8,
            "d2h_bytes_per_step": (m + 9 * n) * 8, "ms_per_step": ms_e2e}
 
@@ -616,6 +620,22 @@ def run_gpu(args, wl):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, **arrays):
+    """DIR/<name>.npy of every array a caller of the timed solve receives, in the layout it receives them (float64),
+    so that two builds can be compared output for output.  Every workload's outputs fit the size limit as a whole."""
+    import numpy as np
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items() if v is not None}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def side_stages(desc_b200, Ind_d, R_d, wl, kw, peak, seed):
     """CEMP / CEMP+GCW / CEMP+MST / MPLS / Spectral (the comparators Demo/compare_algorithms.m runs beside DESC) with
     the demo's parameters on the bench graph; device-timed by the library."""
@@ -663,7 +683,14 @@ def main():
                     help="seconds of CPU work one CPU sample may take (sizes the sample graph)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-side", action="store_true", help="skip the SURVEY 8(f) side stages (CEMP, MPLS, ...)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (S_vec.npy; R_est.npy when the step runs GCW) to DIR; "
+                         "that step also copies them to the host, which the other steps skip")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "desc_b200":
+        ap.error("--dump-outputs writes what the GPU solve returns; the reference arm solves a different graph")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

@@ -36,6 +36,13 @@ def test_reference_arm_ring_workload_has_no_gcw_stage():
     assert j["config"]["same_config"] is False and j["config"]["n"] < 50000
 
 
+def test_step_counts_below_one_are_rejected():
+    for steps in ("0", "-1"):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", steps],
+                           capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert r.returncode == 2 and "--steps" in r.stderr and r.stdout == ""
+
+
 def test_other_ranks_of_a_torchrun_launch_print_nothing():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],
