@@ -161,6 +161,8 @@ struct desc_b200_handle {
     double* w[2] = {nullptr, nullptr};     // n_slots each (ping-pong)
     double* S[2] = {nullptr, nullptr};     // m each
     double* acc[2] = {nullptr, nullptr};   // 2m+2 each: partner sums via min/max endpoint, + [obj, change]
+    double* acc2[2] = {nullptr, nullptr};  // 2m each (streamed path, one GPU): the share of the pass over larger endpoints
+    double* S_adj = nullptr;                // 2m+4 (streamed path): S of the current state in adjacency order
     double* adam_m = nullptr;
     double* adam_v = nullptr;
     int final_buf = 0;                      // which ping-pong buffer holds the result

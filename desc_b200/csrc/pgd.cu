@@ -319,6 +319,10 @@ struct BlkArgs {
     int v0, v1;        // local vertex range
     int tstride;       // padded max degree (table stride)
     double* partial;   // 2 per CTA of k_pgd_block
+    // streamed path only
+    const double* S_adj;   // S of the current state in adjacency order (k_pgd_s_adj)
+    const double* acc2_cur;  // partner sums of the pass over larger endpoints: read by the streamed kernel,
+    double* acc2_next;       //   written by the pass itself (both null on multi-GPU handles: it adds to acc_next)
 };
 
 // shared tables: T_S[tstride] | T_acc[BLK_WARPS][tstride]
@@ -570,6 +574,16 @@ k_pgd_scatter(BlkArgs a, const double* __restrict__ w) {
     blk_flush(a, v, deg, rs, T_acc, a.p.acc_next);
 }
 
+// S in adjacency order, S_adj[p] = S[adj_eid[p]]: the table prologues of both streamed passes then read
+// a vertex's row contiguously instead of gathering it (one 2m-entry L2 gather per state, here)
+__global__ void __launch_bounds__(256)
+k_pgd_s_adj(const int* __restrict__ adj_eid, const double* __restrict__ S, int64_t n2m, const int* __restrict__ ctrl,
+            double* __restrict__ S_adj) {
+    if (ctrl[0]) return;
+    const int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (p < n2m) S_adj[p] = S[adj_eid[p]];
+}
+
 // fixed-order reduction of the per-CTA partials into red[0] (objective) and red[1] (change)
 #define PGD_PART_TB 1024
 __global__ void __launch_bounds__(PGD_PART_TB)
@@ -637,7 +651,7 @@ static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, i
         }
     }
     sa.tsc = (TE * h->max_ns + G * EPL + 16 + 7) & ~7;
-    const size_t fixed = st_fixed_bytes(TE, a.tstride, h->max_ns, NSW), stage = st_stage_bytes(sa.tsc, TE);
+    const size_t fixed = st_fixed_bytes(a.tstride, h->max_ns, NSW), stage = st_stage_bytes(sa.tsc, TE) + st_hdr_bytes(TE);
     // several CTAs per SM: one CTA's table prologue / flush overlaps the others' streaming.
     // 228 KB of shared memory per SM, 1 KB reserved per CTA.
     int nst = 0;
@@ -650,6 +664,8 @@ static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, i
     if (dry) return DESC_B200_OK;
     sa.nstages = nst;
     sa.sjk = h->sjk;
+    sa.S_adj = a.S_adj;
+    sa.acc2_cur = a.acc2_cur;
     const size_t smem = fixed + nst * stage;
     constexpr int NT = (NCW + NSW + 1) * 32;
     if (rule_kind == 0) {
@@ -775,6 +791,14 @@ static int launch_passb(desc_b200_handle* h, const BlkArgs& a, const double* w_t
     }
     if (nw >= 8) PB_LAUNCH(8) else if (nw >= 4) PB_LAUNCH(4) else PB_LAUNCH(2)
 #undef PB_LAUNCH
+    KERNEL_CHECK(h);
+    return DESC_B200_OK;
+}
+
+static int launch_s_adj(desc_b200_handle* h, const double* S) {
+    const int64_t n2m = 2 * h->m;
+    if (n2m == 0) return DESC_B200_OK;
+    k_pgd_s_adj<<<(unsigned)((n2m + 255) / 256), 256, 0, h->stream>>>(h->adj_eid, S, n2m, h->d_ctrl, h->S_adj);
     KERNEL_CHECK(h);
     return DESC_B200_OK;
 }
@@ -1247,6 +1271,9 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
     ba.v1 = h->v_end;
     ba.tstride = (h->maxdeg + 1 + 3) & ~3;   // >= maxdeg + 1: the last entry is a dummy slot for inactive lanes
     ba.partial = h->pgd_partial;
+    ba.S_adj = nullptr;
+    ba.acc2_cur = nullptr;
+    ba.acc2_next = nullptr;
     const size_t smem_blk = (size_t)(1 + BLK_WARPS) * ba.tstride * sizeof(double);
     const size_t smem_sc = (size_t)BLK_WARPS * ba.tstride * sizeof(double);
     const int launches0 = h->launches;
@@ -1255,6 +1282,15 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         stream = h->sjk != nullptr && launch_stream_any(h, ba, adam ? 1 : 0, true) == DESC_B200_OK &&
                  (size_t)(2 + 8) * ba.tstride * sizeof(double) <= 226 * 1024;
     }
+    if (stream) {
+        if (!h->S_adj) CUDA_TRY(cudaMalloc(&h->S_adj, (2 * m + 4) * sizeof(double)));   // +4: 16-byte widened bulk copies
+        ba.S_adj = h->S_adj;
+        // one GPU: the pass over larger endpoints stores its partner sums apart (no read-modify-write of acc)
+        if (h->world == 1)
+            for (int b = 0; b < 2; b++)
+                if (!h->acc2[b]) CUDA_TRY(cudaMalloc(&h->acc2[b], std::max<int64_t>(2 * m, 1) * sizeof(double)));
+    }
+    const bool use_acc2 = stream && h->world == 1;
     const int G = h->max_ns <= 32 ? 8 : (h->max_ns <= 64 ? 16 : 32);
     const int aux_grid = DESC_SMS * 8;
 
@@ -1282,7 +1318,11 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         }
     }
     DESC_TRY(exchange_S(h, 0));
-    if (stream && h->n_slots > 0) DESC_TRY(launch_passb(h, ba, h->w[0]));   // needs every rank's S_0
+    if (stream) DESC_TRY(launch_s_adj(h, h->S[0]));   // needs every rank's S_0
+    if (stream && h->n_slots > 0) {
+        ba.acc2_next = use_acc2 ? h->acc2[0] : nullptr;
+        DESC_TRY(launch_passb(h, ba, h->w[0]));
+    }
     DESC_TRY(exchange_partner_sums(h, 0, false));
 
     // per-iteration kernel timing: events around the iteration kernels only
@@ -1318,12 +1358,18 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         const bool timed = t <= 512;
         if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1)], st));
         if (stream) {
-            // pass 1 (smaller endpoints): update; pass 2 (larger endpoints) needs all of S_t
+            // pass 1 (smaller endpoints): update; pass 2 (larger endpoints) needs all of S_t.  One S_adj serves
+            // pass 2 of iteration t and pass 1 of iteration t+1 (stream order).  It is no output: once the lagged
+            // stop flag is set every later kernel (the relayout too) returns, and the results are read from
+            // the ping-ponged S / w.
             ba.p = a;
+            ba.acc2_cur = use_acc2 ? h->acc2[cur] : nullptr;
+            ba.acc2_next = use_acc2 ? h->acc2[nxt] : nullptr;
             DESC_TRY(launch_stream_any(h, ba, adam ? 1 : 0));
             if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 1], st));
             DESC_TRY(exchange_S(h, nxt));
             if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 2], st));
+            DESC_TRY(launch_s_adj(h, h->S[nxt]));   // timed with pass 2
             DESC_TRY(launch_passb(h, ba, h->w[nxt]));
             k_pgd_partials<<<1, PGD_PART_TB, 0, st>>>(h->pgd_partial, h->v_end - h->v_begin, h->d_ctrl, h->acc[nxt] + 2 * m);
             KERNEL_CHECK(h);

@@ -11,6 +11,11 @@
 // the (w, rank) loads of the next two batches of edges and the headers of the third in flight in
 // registers while it works on the current batch.
 // No atomics: every partner-sum entry (edge, side v) is owned by vertex v's CTA.
+// The S table is a contiguous read of S_adj (S in adjacency order, k_pgd_s_adj).  The partner sums
+// go to acc2_next with plain stores, every entry of the vertex's row in every launch (zeros when the
+// vertex has no local in-edges); the streamed kernel of the next iteration adds them to its own
+// (acc).  Multi-GPU handles (acc2_next null) add them to acc_next instead, so that one exchange
+// reduces the whole sum to the owners.
 #ifndef PB_U
 #define PB_U 4
 #endif
@@ -20,6 +25,16 @@
 #ifndef PB_DEPTH
 #define PB_DEPTH 2                      // batches of (w, rank) loads in flight ahead of the current one
 #endif
+
+// partner-sum entry (edge, side v) of adjacency position rs + r of vertex v
+__device__ __forceinline__ int64_t pb_acc_pos(const BlkArgs& a, int v, int rs, int r) {
+    return 2 * (int64_t)a.adj_eid[rs + r] + (v < a.adj_nbr[rs + r] ? 0 : 1);
+}
+// a vertex without local in-edges: its row of acc2_next is zero in this launch
+__device__ __forceinline__ void pb_zero_row(const BlkArgs& a, int v, int rs, int deg) {
+    if (!a.acc2_next) return;
+    for (int r = threadIdx.x; r < deg; r += blockDim.x) a.acc2_next[pb_acc_pos(a, v, rs, r)] = 0.0;
+}
 
 // PB_WARPS warps (= private tables) per CTA: 8 when a vertex has hundreds of local in-edges, fewer
 // (smaller CTAs, more of them per SM) when sharding over GPUs leaves each CTA little work, so that
@@ -39,27 +54,29 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
     const int rs = a.rowstart[v];
     const int deg = a.rowstart[v + 1] - rs;
     const int ub = min(a.v1, v);                           // neighbours u with v0 <= u < ub
-    if (ub <= a.v0) return;
+    if (ub <= a.v0) {
+        pb_zero_row(a, v, rs, deg);
+        return;
+    }
     const int lo = rs + (a.v0 > 0 ? desc_rank(a.bm, a.bmprefix, a.nwords, v, a.v0) : 0);
     const int hi = rs + desc_rank(a.bm, a.bmprefix, a.nwords, v, ub);
-    if (hi <= lo) return;
+    if (hi <= lo) {
+        pb_zero_row(a, v, rs, deg);
+        return;
+    }
     int2* shdr = reinterpret_cast<int2*>(T_acc + (size_t)PB_WARPS * a.tstride);   // headers of the in-edges [lo, hi)
-    // table prologue, KU entries per thread at a time: all index loads, then all S gathers, in flight
-    // together (a plain loop serialises two dependent global latencies per trip)
+    // table prologue, KU entries per thread at a time: all loads in flight together
     // (KU grows as the CTA shrinks: a 2-warp CTA - multi-GPU shards - still covers ~1280 entries per trip)
     constexpr int KU = 40 / PB_WARPS;
     for (int rb = threadIdx.x; rb < deg; rb += PB_TB * KU) {
-        int e2[KU];
         double sv[KU];
         int2 hv[KU];
 #pragma unroll
         for (int k = 0; k < KU; k++) {
             const int r = rb + k * PB_TB;
-            e2[k] = r < deg ? a.adj_eid[rs + r] : -1;
+            sv[k] = (WRITE_SJK && r < deg) ? a.S_adj[rs + r] : 0.0;
             hv[k] = lo + r < hi ? __ldg(jhdr + lo + r) : make_int2(0, 0);
         }
-#pragma unroll
-        for (int k = 0; k < KU; k++) sv[k] = (WRITE_SJK && e2[k] >= 0) ? a.p.S_next[e2[k]] : 0.0;
 #pragma unroll
         for (int k = 0; k < KU; k++) {
             const int r = rb + k * PB_TB;
@@ -167,18 +184,18 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
     }
     __syncthreads();
     // flush (every entry (edge, side v) is owned by this CTA within this kernel), KU entries per
-    // thread at a time so that the index loads and the read-modify-writes overlap
+    // thread at a time so that the index loads (and, multi-GPU, the read-modify-writes) overlap
+    double* const out = a.acc2_next ? a.acc2_next : a.p.acc_next;
     for (int rb = threadIdx.x; rb < deg; rb += PB_TB * KU) {
         int64_t pos[KU];
         double old[KU];
 #pragma unroll
         for (int k = 0; k < KU; k++) {
             const int r = rb + k * PB_TB;
-            pos[k] = -1;
-            if (r < deg) pos[k] = 2 * (int64_t)a.adj_eid[rs + r] + (v < a.adj_nbr[rs + r] ? 0 : 1);
+            pos[k] = r < deg ? pb_acc_pos(a, v, rs, r) : -1;
         }
 #pragma unroll
-        for (int k = 0; k < KU; k++) old[k] = pos[k] >= 0 ? a.p.acc_next[pos[k]] : 0.0;
+        for (int k = 0; k < KU; k++) old[k] = (!a.acc2_next && pos[k] >= 0) ? a.p.acc_next[pos[k]] : 0.0;
 #pragma unroll
         for (int k = 0; k < KU; k++) {
             const int r = rb + k * PB_TB;
@@ -186,7 +203,7 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
                 double x = 0.0;
 #pragma unroll
                 for (int q = 0; q < PB_WARPS; q++) x += T_acc[q * a.tstride + r];
-                a.p.acc_next[pos[k]] = old[k] + x;
+                out[pos[k]] = a.acc2_next ? x : old[k] + x;
             }
         }
     }
@@ -239,10 +256,16 @@ k_pgd_passb_tma(PassbArgs pa) {
     const int rs = a.rowstart[v];
     const int deg = a.rowstart[v + 1] - rs;
     const int ub = min(a.v1, v);                           // neighbours u with v0 <= u < ub
-    if (ub <= a.v0) return;
+    if (ub <= a.v0) {
+        pb_zero_row(a, v, rs, deg);
+        return;
+    }
     const int lo = rs + (a.v0 > 0 ? desc_rank(a.bm, a.bmprefix, a.nwords, v, a.v0) : 0);
     const int hi = rs + desc_rank(a.bm, a.bmprefix, a.nwords, v, ub);
-    if (hi <= lo) return;
+    if (hi <= lo) {
+        pb_zero_row(a, v, rs, deg);
+        return;
+    }
     const int ntiles = (hi - lo + PT_TE - 1) / PT_TE;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (threadIdx.x == 0) {
@@ -291,7 +314,7 @@ k_pgd_passb_tma(PassbArgs pa) {
         // ------------------------------------------------------------------ scatter warps
         constexpr int NT = PT_NSW * 32;
         for (int r = threadIdx.x; r < deg; r += NT) {
-            T_S[r] = a.p.S_next[a.adj_eid[rs + r]];
+            T_S[r] = a.S_adj[rs + r];
 #pragma unroll
             for (int q = 0; q < PT_NSW; q++) T_acc[q * a.tstride + r] = 0.0;
         }
@@ -356,8 +379,10 @@ k_pgd_passb_tma(PassbArgs pa) {
         double x = 0.0;
 #pragma unroll
         for (int q = 0; q < PT_NSW; q++) x += T_acc[q * a.tstride + r];
-        const int e2 = a.adj_eid[rs + r];
-        const int k = a.adj_nbr[rs + r];
-        a.p.acc_next[2 * (int64_t)e2 + (v < k ? 0 : 1)] += x;   // owned by this CTA within this kernel
+        const int64_t pos = pb_acc_pos(a, v, rs, r);   // owned by this CTA within this kernel
+        if (a.acc2_next)
+            a.acc2_next[pos] = x;
+        else
+            a.p.acc_next[pos] += x;
     }
 }

@@ -8,7 +8,9 @@
 //     arrays (w, S0, sjk, rk_i: contiguous because the edges of a vertex block and their slot
 //     lists are contiguous) and per-edge arrays (rowptr, partner sums, S) into a ring of shared-
 //     memory stages; completion is signalled on an mbarrier (complete_tx::bytes).  L2 policy
-//     evict_first for the slot streams: they must not evict S.
+//     evict_first for the slot streams: they must not evict S.  Before the first tile it copies the
+//     vertex's S table, S_adj[rowstart[v] .. rowstart[v+1]) (S in adjacency order, k_pgd_s_adj),
+//     with one more bulk copy on its own mbarrier: no index-dependent gather in the prologue.
 //   * COMPUTE warps: G lanes own one edge and keep EPL slots each in registers.  They read the
 //     stage, compute gradient / step / projection, write w_t in place into the stage, publish
 //     (slot offset, count) of their edges and arrive on the stage's `done` mbarrier.  There is NO
@@ -94,22 +96,26 @@ struct StreamArgs {
     int tsc;          // slot capacity of one stage (multiple of 8)
     int max_ns;       // longest slot list (size of the reciprocal table)
     const double* sjk;  // S[e_jk] per slot for the current state (pgd_passb.cuh)
+    const double* S_adj;    // S_cur in adjacency order (2m + 4: 16-byte widened bulk copy)
+    const double* acc2_cur; // partner sums of the pass over larger endpoints (2m), null on multi-GPU handles
     long long* trace; // DESC_B200_TRACE: per-tile event clocks of one CTA (null = off)
     int trace_cta;
 };
 #define ST_TRACE(k, t) \
     do { if (sa.trace && (int)blockIdx.x == sa.trace_cta && (t) < 64 && lane == 0) sa.trace[(t) * 8 + (k)] = clock64(); } while (0)
 
-// shared-memory carve-up: barriers | per-stage edge headers | 1/c table | T_S | T_acc[NSW] | stages.
+// shared-memory carve-up: barriers | edge headers[nstages][TE] | 1/c table | T_S[tstride+2] | T_acc[NSW] | stages.
 // One stage: w[tsc] f64 | S0[tsc] f64 | sjk[tsc] f64 | rk_i[tsc] u16 | rowptr[TE+2] i64 |
-//            acc_cur[2*TE] f64 | S_cur[TE+2] f64          (every offset a multiple of 16 bytes)
+//            acc_cur[2*TE] f64 | acc2_cur[2*TE] f64 | S_cur[TE+2] f64   (every offset a multiple of 16 bytes)
+// The edge headers of a stage (st_hdr_bytes) sit apart from its ring slot, so only the stages in use take room.
 __host__ __device__ __forceinline__ size_t st_stage_bytes(int tsc, int te) {
-    return (size_t)tsc * (8 + 8 + 8 + 2) + (size_t)(te + 2) * 8 + (size_t)te * 16 + (size_t)(te + 2) * 8;
+    return (size_t)tsc * (8 + 8 + 8 + 2) + (size_t)(te + 2) * 8 + (size_t)te * 32 + (size_t)(te + 2) * 8;
 }
+__host__ __device__ __forceinline__ size_t st_hdr_bytes(int te) { return (size_t)te * sizeof(int2); }
 __host__ __device__ __forceinline__ size_t st_rcp_bytes(int max_ns) { return ((size_t)(max_ns + 1) * 8 + 15) & ~(size_t)15; }
-__host__ __device__ __forceinline__ size_t st_fixed_bytes(int te, int tstride, int max_ns, int nsw) {
-    return 128 + (size_t)ST_MAXSTAGES * te * sizeof(int2) + st_rcp_bytes(max_ns) +
-           (size_t)(1 + ST_TPW * nsw) * tstride * sizeof(double);   // T_S + the scatter warps' private tables
+__host__ __device__ __forceinline__ size_t st_fixed_bytes(int tstride, int max_ns, int nsw) {
+    return 128 + st_rcp_bytes(max_ns) +
+           (size_t)(1 + ST_TPW * nsw) * tstride * sizeof(double) + 16;   // T_S (+2: widened copy) + the scatter warps' private tables
 }
 
 // G lanes per edge with EPL slots each, NCW compute warps, ST_NSW scatter warps (private tables),
@@ -126,16 +132,18 @@ k_pgd_stream(StreamArgs sa) {
     uint64_t* full = bars;
     uint64_t* done = bars + ST_MAXSTAGES;
     uint64_t* empty = bars + 2 * ST_MAXSTAGES;
+    uint64_t* tbar = bars + 3 * ST_MAXSTAGES;   // the S table
     int2* hdr = reinterpret_cast<int2*>(smem_raw + 128);
-    double* rcp = reinterpret_cast<double*>(smem_raw + 128 + (size_t)ST_MAXSTAGES * TE * sizeof(int2));
-    double* T_S = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(rcp) + st_rcp_bytes(sa.max_ns));
-    double* T_acc = T_S + a.tstride;
+    double* rcp = reinterpret_cast<double*>(smem_raw + 128 + (size_t)sa.nstages * st_hdr_bytes(TE));
+    double* T_S0 = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(rcp) + st_rcp_bytes(sa.max_ns));
+    double* T_acc = T_S0 + a.tstride + 2;
     constexpr int NTAB = ST_TPW * ST_NSW;
     unsigned char* stage0 = reinterpret_cast<unsigned char*>(T_acc + (size_t)NTAB * a.tstride);
     const int tsc = sa.tsc;
     const size_t stage_bytes = st_stage_bytes(tsc, TE);
     const size_t off_d = (size_t)tsc * 8, off_sj = (size_t)tsc * 16, off_rk = (size_t)tsc * 24;
-    const size_t off_rp = (size_t)tsc * 26, off_acc = off_rp + (size_t)(TE + 2) * 8, off_so = off_acc + (size_t)TE * 16;
+    const size_t off_rp = (size_t)tsc * 26, off_acc = off_rp + (size_t)(TE + 2) * 8, off_acc2 = off_acc + (size_t)TE * 16;
+    const size_t off_so = off_acc2 + (size_t)TE * 16;
     const int NST = sa.nstages;
 
     const int v = a.v0 + blockIdx.x;
@@ -157,12 +165,14 @@ k_pgd_stream(StreamArgs sa) {
     }
     const int ntiles = (e_hi - e_lo + TE - 1) / TE;
     const int eoff = e_lo & 1;   // the per-edge arrays are copied from an even edge index (16-byte alignment)
+    const double* T_S = T_S0 + (rs & 1);   // the same for the S table: copied from an even adjacency position
     if (threadIdx.x == 0) {
         for (int s = 0; s < NST; s++) {
             mbar_init(&full[s], 1);
             mbar_init(&done[s], NCW);
             mbar_init(&empty[s], ST_NSW);
         }
+        mbar_init(tbar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
@@ -173,6 +183,11 @@ k_pgd_stream(StreamArgs sa) {
         // ------------------------------------------------------------------ producer
         // lanes prefetch the slot boundaries of 32 tiles at a time; lane 0 issues the bulk copies
         const uint64_t pol = l2_evict_first_policy();
+        if (lane == 0) {   // the S table first: its latency overlaps the ring fill
+            const int p0 = rs & ~1, cnt = ((rs + deg + 1) & ~1) - p0;
+            mbar_expect_tx(tbar, (uint32_t)(cnt * 8));
+            bulk_g2s_plain(T_S0, sa.S_adj + p0, (uint32_t)(cnt * 8), tbar);
+        }
         int s = 0;
         uint32_t ph = 0;
         for (int tb = 0; tb < ntiles; tb += 32) {
@@ -208,9 +223,11 @@ k_pgd_stream(StreamArgs sa) {
                     ST_TRACE(0, t);
                     mbar_wait(&empty[s], ph ^ 1u);
                     ST_TRACE(1, t);
-                    mbar_expect_tx(&full[s], (uint32_t)(cnt * 26 + rp_cnt * 8 + (e1 - e0) * 16 + so_cnt * 8));
+                    mbar_expect_tx(&full[s], (uint32_t)(cnt * 26 + rp_cnt * 8 + (e1 - e0) * (sa.acc2_cur ? 32 : 16) + so_cnt * 8));
                     bulk_g2s_plain(st + off_rp, a.p.rowptr + e0a, (uint32_t)(rp_cnt * 8), &full[s]);
                     bulk_g2s_plain(st + off_acc, a.p.acc_cur + 2 * (int64_t)e0, (uint32_t)((e1 - e0) * 16), &full[s]);
+                    if (sa.acc2_cur)
+                        bulk_g2s_plain(st + off_acc2, sa.acc2_cur + 2 * (int64_t)e0, (uint32_t)((e1 - e0) * 16), &full[s]);
                     bulk_g2s_plain(st + off_so, a.p.S_cur + e0a, (uint32_t)(so_cnt * 8), &full[s]);
                     if (cnt > 0) {
                         bulk_g2s(st, a.p.w_cur + base, (uint32_t)(cnt * 8), &full[s], pol);
@@ -230,27 +247,13 @@ k_pgd_stream(StreamArgs sa) {
         // ------------------------------------------------------------------ tables (compute + scatter warps)
         constexpr int NT = (NCW + ST_NSW) * 32;
         for (int c = threadIdx.x; c <= sa.max_ns; c += NT) rcp[c] = c > 0 ? 1.0 / (double)c : 0.0;
-        // KU entries per thread at a time: index loads, then S gathers, all in flight together
-        constexpr int KU = 4;
-        for (int rb = threadIdx.x; rb < deg; rb += NT * KU) {
-            int e2[KU];
-            double sv[KU];
+        for (int r = threadIdx.x; r < deg; r += NT) {
 #pragma unroll
-            for (int k = 0; k < KU; k++) e2[k] = rb + k * NT < deg ? a.adj_eid[rs + rb + k * NT] : -1;
-#pragma unroll
-            for (int k = 0; k < KU; k++) sv[k] = e2[k] >= 0 ? a.p.S_cur[e2[k]] : 0.0;
-#pragma unroll
-            for (int k = 0; k < KU; k++) {
-                const int r = rb + k * NT;
-                if (r < deg) {
-                    T_S[r] = sv[k];
-#pragma unroll
-                    for (int q = 0; q < NTAB; q++) T_acc[q * a.tstride + r] = 0.0;
-                }
-            }
+            for (int q = 0; q < NTAB; q++) T_acc[q * a.tstride + r] = 0.0;
         }
         asm volatile("bar.sync 1, %0;" ::"n"(NT) : "memory");
         if (warp < NCW) {
+            mbar_wait(tbar, 0);   // the S table has arrived
             // -------------------------------------------------------------- compute
             // Branch-free inner loop: a lane's EPL slots are idx = r + x*G; lanes past the end of the
             // slot list read harmless stage bytes and are neutralised with selects.
@@ -282,6 +285,11 @@ k_pgd_stream(StreamArgs sa) {
                     const double2 ab = reinterpret_cast<const double2*>(st + off_acc)[q];
                     A = ab.x;
                     B = ab.y;
+                    if (sa.acc2_cur) {   // x1 + x2: the sum the read-modify-write of the multi-GPU flush forms
+                        const double2 ab2 = reinterpret_cast<const double2*>(st + off_acc2)[q];
+                        A = ab.x + ab2.x;
+                        B = ab.y + ab2.y;
+                    }
                     Sold = (reinterpret_cast<const double*>(st + off_so) + eoff)[q];
                 }
                 const int nx = (ns - r + G - 1) / G;   // this lane owns slots x < nx  (G is a power of two)
@@ -508,7 +516,8 @@ k_pgd_stream(StreamArgs sa) {
     __syncthreads();
     if (warp == 0) ST_TRACE(6, 1);
     // flush the private tables: every (edge, side) entry belongs to exactly one vertex block, and this
-    // kernel is the first writer of acc_next in an iteration => plain stores (k_pgd_scatter adds later)
+    // kernel is the first writer of acc_next in an iteration => plain stores (the pass over larger
+    // endpoints stores its share into acc2_next, or adds it here on multi-GPU handles)
     {
         constexpr int KU = 4;
         for (int rb = threadIdx.x; rb < deg; rb += NTHREADS * KU) {
