@@ -74,9 +74,8 @@ void desc_b200_destroy(desc_b200_handle* h) {
                     h->d_ctrl_f, h->omega, h->isd, h->X[0], h->X[1], h->gcw_coef, h->gcw_red,
                     h->gcw_small, h->gcw_res, h->R_est, h->d_err, h->d_Sin, h->rk_i, h->rk_j, h->estart,
                     h->pgd_partial, h->jhdr, h->sjk, h->thr_key, h->thr_k, h->comm_scratch,
-                    h->cemp_S[0], h->cemp_S[1], h->diag_work, h->diag_hist, h->R_mst, h->ell_vtile, h->ell_tiles,
-                    h->ell_tcnt, h->ell_d, h->ell_rk, h->ell_pj, h->ell_w[0], h->ell_w[1], h->ell_adam_m, h->ell_adam_v,
-                    h->gcw_coef_adj, h->acc2[0], h->acc2[1], h->S_adj};
+                    h->cemp_S[0], h->cemp_S[1], h->diag_work, h->diag_hist, h->R_mst, h->gcw_coef_adj, h->acc2[0],
+                    h->acc2[1], h->S_adj};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (h->h_ctrl) cudaFreeHost(h->h_ctrl);

@@ -944,22 +944,8 @@ static void free_incidence(desc_b200_handle* h) {
     h->rk_i = h->rk_j = nullptr;
     h->jhdr = nullptr;
     h->sjk = nullptr;
-    {
-        void* ell[] = {h->ell_vtile, h->ell_tiles, h->ell_tcnt, h->ell_d, h->ell_rk, h->ell_pj, h->ell_w[0], h->ell_w[1],
-                       h->ell_adam_m, h->ell_adam_v};
-        for (void* p : ell) cudaFree(p);
-        h->ell_vtile = h->ell_tcnt = nullptr;
-        h->ell_tiles = nullptr;
-        h->ell_d = h->ell_w[0] = h->ell_w[1] = h->ell_adam_m = h->ell_adam_v = nullptr;
-        h->ell_rk = nullptr;
-        h->ell_pj = nullptr;
-        h->ell_G = 0;
-        h->ell_ntiles = 0;
-        h->ell_size = 0;
-        h->ell_have_d = false;
-        h->adam_valid = false;
-        h->has_dup_apex = false;
-    }
+    h->adam_valid = false;
+    h->has_dup_apex = false;
     for (int b = 0; b < 2; b++) {
         cudaFree(h->w[b]);
         h->w[b] = nullptr;

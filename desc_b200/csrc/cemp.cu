@@ -16,15 +16,13 @@
 // + 8*m (rowptr) + 8*m (vector out).  HBM-bound; no tensor cores.
 #include "internal.cuh"
 
-#include <stdlib.h>
-
 #include <algorithm>
 
-// Edge distribution: BLOCKED gives every CTA one contiguous run of edges instead of a grid-stride.  Edges are
-// (i,j)-sorted, so a CTA then works through whole vertex blocks, and the x[] entries of the edges (i,k), k>i -- two
-// thirds of the "via i" gathers -- are the CTA's own few-KB range and stay in L1 instead of costing an L2 sector each
-// (the kernel is bound by L2 sector throughput: 7.7e8 sectors = 10 TB/s at 2.4 ms, profiles/r01_cemp_ncu_summary.txt).
-template <int G, bool BLOCKED>
+// Edge distribution: every CTA takes one contiguous run of edges instead of a grid-stride.  Edges are (i,j)-sorted, so
+// a CTA then works through whole vertex blocks, and the x[] entries of the edges (i,k), k>i -- two thirds of the "via i"
+// gathers -- are the CTA's own few-KB range and stay in L1 instead of costing an L2 sector each (the kernel is bound by
+// L2 sector throughput: 7.7e8 sectors = 10 TB/s at 2.4 ms, profiles/r01_cemp_ncu_summary.txt).
+template <int G>
 __global__ void __launch_bounds__(256)
 k_cemp_reweight(const int64_t* __restrict__ rowptr, const uint32_t* __restrict__ pk_jk,
                 const uint32_t* __restrict__ pk_ki, const double* __restrict__ S0,
@@ -32,17 +30,10 @@ k_cemp_reweight(const int64_t* __restrict__ rowptr, const uint32_t* __restrict__
                 int64_t slot_base, double beta, double empty_value) {
     const int r = threadIdx.x & (G - 1);
     const int sub = (threadIdx.x & 31) / G;
-    int64_t first, last, step;
-    if (BLOCKED) {
-        const int64_t per = (e1 - e0 + gridDim.x - 1) / gridDim.x;
-        first = e0 + blockIdx.x * per + (threadIdx.x >> 5) * (32 / G);   // first group of this warp
-        last = min(e1, e0 + (blockIdx.x + 1) * per);
-        step = blockDim.x / G;
-    } else {
-        first = e0 + (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / G - sub;
-        last = e1;
-        step = ((int64_t)gridDim.x * blockDim.x) / G;
-    }
+    const int64_t per = (e1 - e0 + gridDim.x - 1) / gridDim.x;
+    const int64_t first = e0 + blockIdx.x * per + (threadIdx.x >> 5) * (32 / G);   // first group of this warp
+    const int64_t last = min(e1, e0 + (blockIdx.x + 1) * per);
+    const int64_t step = blockDim.x / G;
     // the trip count is warp-uniform (shuffles below): every lane of a warp iterates from the warp's first group
     for (int64_t eb = first; eb < last; eb += step) {
         const int64_t e = eb + sub;
@@ -72,18 +63,9 @@ int desc_cemp_reweight(desc_b200_handle* h, const double* x_cur, double* x_next,
     if (h->e_end > h->e_begin) {
         const int grid = DESC_SMS * 8;
         cudaStream_t st = h->stream;
-        // DESC_B200_CEMP_DIST = stride | block (default): kernel-tuning switch, same arithmetic either way
-        const char* dist = getenv("DESC_B200_CEMP_DIST");
-        const bool blocked = !(dist && strcmp(dist, "stride") == 0);
-#define CEMP_LAUNCH(G)                                                                                              \
-    do {                                                                                                            \
-        if (blocked)                                                                                                \
-            k_cemp_reweight<G, true><<<grid, 256, 0, st>>>(h->rowptr, h->pk_jk, h->pk_ki, h->S0, x_cur, x_next,     \
-                                                           h->e_begin, h->e_end, h->slot_base, beta, empty_value); \
-        else                                                                                                        \
-            k_cemp_reweight<G, false><<<grid, 256, 0, st>>>(h->rowptr, h->pk_jk, h->pk_ki, h->S0, x_cur, x_next,    \
-                                                            h->e_begin, h->e_end, h->slot_base, beta, empty_value); \
-    } while (0)
+#define CEMP_LAUNCH(G)                                                                                        \
+    k_cemp_reweight<G><<<grid, 256, 0, st>>>(h->rowptr, h->pk_jk, h->pk_ki, h->S0, x_cur, x_next, h->e_begin, \
+                                             h->e_end, h->slot_base, beta, empty_value)
         if (h->max_ns <= 8)
             CEMP_LAUNCH(8);
         else if (h->max_ns <= 16)

@@ -29,7 +29,6 @@ struct NcclApi {
     ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*Broadcast)(const void*, void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*ReduceScatter)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*GroupStart)() = nullptr;
@@ -62,7 +61,6 @@ int nccl_load() {
     LOAD(AllReduce, "ncclAllReduce");
     LOAD(Broadcast, "ncclBroadcast");
     LOAD(AllGather, "ncclAllGather");
-    LOAD(ReduceScatter, "ncclReduceScatter");
     LOAD(Send, "ncclSend");
     LOAD(Recv, "ncclRecv");
     LOAD(GroupStart, "ncclGroupStart");
@@ -151,20 +149,7 @@ int desc_allreduce_sum(desc_b200_handle* h, double* buf, int64_t count) {
     return DESC_B200_OK;
 }
 
-// ---- the two per-iteration exchanges as NCCL collectives on padded, rank-major staging -------------------------
-// The shards are ragged (vertex-aligned edge ranges), NCCL's all-gather / reduce-scatter want equal counts: pack the
-// ranges into slots of the largest range's size, run ONE collective (NVSwitch: ring / NVLS inside NCCL, all links
-// busy), unpack.  Measured on 8 B200 at cfg 4 it is SLOWER than the grouped point-to-point version below (0.41 vs
-// 0.35 ms of exchanges per iteration: the pack / unpack passes cost more than the collectives save), so it is only
-// used with DESC_B200_COMM=coll.  Default: peer-memory stores (end of this file) when CUDA IPC works, else p2p.
-static bool use_collectives(size_t staging_bytes) {
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("DESC_B200_COMM");
-        mode = (e && strcmp(e, "coll") == 0) ? 1 : 0;
-    }
-    return mode == 1 && staging_bytes <= ((size_t)1 << 30);
-}
+// receive buffer of desc_reduce_to_owners, grown to `need` bytes
 static int comm_scratch_need(desc_b200_handle* h, size_t need) {
     if (h->comm_scratch_bytes < need) {
         if (h->comm_scratch) cudaFree(h->comm_scratch);
@@ -175,47 +160,6 @@ static int comm_scratch_need(desc_b200_handle* h, size_t need) {
     }
     return DESC_B200_OK;
 }
-struct RangeTab {
-    int64_t b[65];
-    int world;
-};
-// words of 4 bytes: dst slot r (stride words) <- src range r, or back (pack = 1: ranges -> slots)
-__global__ void k_pack_ranges(uint32_t* __restrict__ slots, uint32_t* __restrict__ flat, RangeTab t, int64_t stride,
-                              int words_per_elem, int pack, int only, int skip) {
-    const int r = blockIdx.y;
-    if ((only >= 0 && r != only) || r == skip) return;
-    const int64_t n = (t.b[r + 1] - t.b[r]) * words_per_elem;
-    uint32_t* f = flat + t.b[r] * words_per_elem;
-    uint32_t* s = slots + r * stride;
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        if (pack)
-            s[i] = f[i];
-        else
-            f[i] = s[i];
-    }
-}
-
-static int allgather_collective(desc_b200_handle* h, void* buf, size_t elem_bytes, const std::vector<int64_t>& bounds) {
-    const int W = h->world, me = h->rank;
-    int64_t maxr = 0;
-    for (int r = 0; r < W; r++) maxr = std::max<int64_t>(maxr, bounds[r + 1] - bounds[r]);
-    if (maxr == 0) return DESC_B200_OK;
-    const int wpe = (int)(elem_bytes / 4);
-    const int64_t stride = maxr * wpe;                           // words per slot
-    DESC_TRY(comm_scratch_need(h, (size_t)W * stride * 4));
-    uint32_t* st = (uint32_t*)h->comm_scratch;
-    RangeTab t;
-    t.world = W;
-    for (int r = 0; r <= W; r++) t.b[r] = bounds[r];
-    dim3 g(DESC_SMS * 2, W);
-    k_pack_ranges<<<g, 256, 0, h->stream>>>(st, (uint32_t*)buf, t, stride, wpe, 1, me, -1);
-    KERNEL_CHECK(h);
-    NCCL_TRY(g_nccl.AllGather(st + (int64_t)me * stride, st, (size_t)stride, ncclUint32, (ncclComm_t)h->comm, h->stream));
-    k_pack_ranges<<<g, 256, 0, h->stream>>>(st, (uint32_t*)buf, t, stride, wpe, 0, -1, me);
-    KERNEL_CHECK(h);
-    h->collectives++;
-    return DESC_B200_OK;
-}
 
 // in-place ragged all-gather: rank r owns elements [bounds[r], bounds[r+1]) of buf.  Point-to-point
 // sends/receives in one group (all pairs move concurrently over NVSwitch) instead of `world`
@@ -223,12 +167,6 @@ static int allgather_collective(desc_b200_handle* h, void* buf, size_t elem_byte
 int desc_allgather_ranges(desc_b200_handle* h, void* buf, size_t elem_bytes,
                           const std::vector<int64_t>& bounds) {
     if (h->world <= 1) return DESC_B200_OK;
-    {
-        int64_t maxr = 0;
-        for (int r = 0; r < h->world; r++) maxr = std::max<int64_t>(maxr, bounds[r + 1] - bounds[r]);
-        if (elem_bytes % 4 == 0 && h->world <= 64 && use_collectives((size_t)h->world * maxr * elem_bytes))
-            return allgather_collective(h, buf, elem_bytes, bounds);
-    }
     const int me = h->rank;
     char* mine = (char*)buf + (size_t)bounds[me] * elem_bytes;
     const size_t my_bytes = (size_t)(bounds[me + 1] - bounds[me]) * elem_bytes;
@@ -264,76 +202,16 @@ __global__ void k_sum_partials(double* __restrict__ own, const double* __restric
     }
     own[i] = acc;
 }
-// the same for 64-bit fixed-point partials (pgd_ell.cuh): integer sums, any order gives the same bits
-__global__ void k_sum_partials_u64(unsigned long long* __restrict__ own, const unsigned long long* __restrict__ scratch,
-                                   int64_t count, int64_t stride, int world) {
-    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i >= count) return;
-    unsigned long long acc = own[i];
-    for (int r = 0; r < world - 1; r++) acc += scratch[(int64_t)r * stride + i];
-    own[i] = acc;
-}
-
-// slots for the reduce-scatter: slot r = [range r of buf (width doubles per element), zero padding, the `tail` doubles]
-// -- every rank puts its tail partial into EVERY slot, so each rank receives the tail's sum with its own range
-__global__ void k_pack_reduce(double* __restrict__ slots, const double* __restrict__ buf, RangeTab t, int64_t stride,
-                              int width, int tail) {
-    const int r = blockIdx.y;
-    const int64_t n = (t.b[r + 1] - t.b[r]) * width;
-    const double* f = buf + t.b[r] * width;
-    double* s = slots + r * stride;
-    const int64_t body = stride - tail;
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < stride; i += (int64_t)gridDim.x * blockDim.x)
-        s[i] = i < n ? f[i] : (i >= body ? buf[t.b[t.world] * width + (i - body)] : 0.0);
-}
-__global__ void k_unpack_reduce(const double* __restrict__ recv, double* __restrict__ buf, int64_t begin, int64_t n,
-                                int64_t body, int64_t tail_at, int tail) {
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n + tail; i += (int64_t)gridDim.x * blockDim.x) {
-        if (i < n)
-            buf[begin + i] = recv[i];
-        else
-            buf[tail_at + (i - n)] = recv[body + (i - n)];
-    }
-}
 
 int desc_reduce_to_owners(desc_b200_handle* h, double* buf, int width, const std::vector<int64_t>& bounds,
-                          int tail, bool body_u64) {
+                          int tail) {
     if (h->world <= 1) return DESC_B200_OK;
     const int me = h->rank, W = h->world;
-    if (!body_u64 && W <= 64) {
-        int64_t mx = 0;
-        for (int r = 0; r < W; r++) mx = std::max<int64_t>(mx, bounds[r + 1] - bounds[r]);
-        const int64_t stride = mx * width + tail;
-        if (use_collectives((size_t)(W + 1) * stride * sizeof(double))) {
-            DESC_TRY(comm_scratch_need(h, (size_t)(W + 1) * stride * sizeof(double)));
-            double* send = (double*)h->comm_scratch;
-            double* recv = send + (int64_t)W * stride;
-            RangeTab t;
-            t.world = W;
-            for (int r = 0; r <= W; r++) t.b[r] = bounds[r];
-            dim3 g(DESC_SMS * 2, W);
-            k_pack_reduce<<<g, 256, 0, h->stream>>>(send, buf, t, stride, width, tail);
-            KERNEL_CHECK(h);
-            NCCL_TRY(g_nccl.ReduceScatter(send, recv, (size_t)stride, ncclFloat64, ncclSum, (ncclComm_t)h->comm, h->stream));
-            const int64_t n = (bounds[me + 1] - bounds[me]) * width;
-            k_unpack_reduce<<<DESC_SMS * 2, 256, 0, h->stream>>>(recv, buf, bounds[me] * width, n, stride - tail,
-                                                                bounds[W] * width, tail);
-            KERNEL_CHECK(h);
-            h->collectives++;
-            return DESC_B200_OK;
-        }
-    }
     const int64_t total = bounds[W];
     int64_t maxr = 0;
     for (int r = 0; r < W; r++) maxr = std::max<int64_t>(maxr, bounds[r + 1] - bounds[r]);
     const int64_t stride = maxr * width + tail;            // doubles per received partial
-    const size_t need = (size_t)(W - 1) * stride * sizeof(double);
-    if (h->comm_scratch_bytes < need) {
-        if (h->comm_scratch) cudaFree(h->comm_scratch);
-        h->comm_scratch = nullptr;
-        CUDA_TRY(cudaMalloc(&h->comm_scratch, need));
-        h->comm_scratch_bytes = need;
-    }
+    DESC_TRY(comm_scratch_need(h, (size_t)(W - 1) * stride * sizeof(double)));
     double* scratch = (double*)h->comm_scratch;
     const int64_t my_cnt = (bounds[me + 1] - bounds[me]) * width;
     NCCL_TRY(g_nccl.GroupStart());
@@ -358,12 +236,8 @@ int desc_reduce_to_owners(desc_b200_handle* h, double* buf, int width, const std
     }
     NCCL_TRY(g_nccl.GroupEnd());
     if (my_cnt > 0) {
-        if (body_u64)
-            k_sum_partials_u64<<<(unsigned)((my_cnt + 255) / 256), 256, 0, h->stream>>>(
-                (unsigned long long*)(buf + bounds[me] * width), (const unsigned long long*)scratch, my_cnt, stride, W);
-        else
-            k_sum_partials<<<(unsigned)((my_cnt + 255) / 256), 256, 0, h->stream>>>(buf + bounds[me] * width, scratch, my_cnt,
-                                                                                  stride, W, me);
+        k_sum_partials<<<(unsigned)((my_cnt + 255) / 256), 256, 0, h->stream>>>(buf + bounds[me] * width, scratch, my_cnt,
+                                                                              stride, W, me);
         KERNEL_CHECK(h);
     }
     if (tail > 0) {
@@ -406,6 +280,10 @@ constexpr size_t SYM_FLAG_BYTES = 2 * 64 * sizeof(uint64_t);
 
 struct PeerPtrs {
     unsigned char* p[64];
+};
+struct RangeTab {
+    int64_t b[65];
+    int world;
 };
 
 __global__ void k_sym_barrier(PeerPtrs pp, int me, int W, unsigned long long epoch, int* __restrict__ err) {
@@ -495,7 +373,7 @@ int sym_barrier(desc_b200_handle* h, SymRegion* R) {
 int desc_sym_setup(desc_b200_handle* h, int64_t m, const std::vector<int64_t>& bounds) {
     if (h->sym) return DESC_B200_OK;   // this handle already uses the region (its sizes do not change)
     if (h->world <= 1 || h->world > 64) return DESC_B200_OK;
-    {
+    {   // DESC_B200_COMM = peer (default) | p2p: any value but peer exchanges through NCCL point-to-point
         const char* e = getenv("DESC_B200_COMM");
         if (e && strcmp(e, "peer") != 0) return DESC_B200_OK;
     }
@@ -625,7 +503,7 @@ int desc_sym_reduce_to_owners(desc_b200_handle* h, double* buf, const std::vecto
     {   // a re-built incidence may have moved the shard boundaries: larger ranges than the scratch go through NCCL
         int64_t maxr = 0;
         for (int r = 0; r < W; r++) maxr = std::max<int64_t>(maxr, bounds[r + 1] - bounds[r]);
-        if (maxr * 2 + 2 > R->cap_stride) return desc_reduce_to_owners(h, buf, 2, bounds, 2, false);
+        if (maxr * 2 + 2 > R->cap_stride) return desc_reduce_to_owners(h, buf, 2, bounds, 2);
     }
     PeerPtrs pp;
     for (int q = 0; q < W; q++) pp.p[q] = R->peer[q];

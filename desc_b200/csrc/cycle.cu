@@ -131,6 +131,5 @@ int desc_cycle_impl(desc_b200_handle* h) {
         KERNEL_CHECK(h);
     }
     h->have_s0 = true;
-    h->ell_have_d = false;   // the lane-per-edge PGD layout re-reads S0 at its next call
     return DESC_B200_OK;
 }

@@ -139,24 +139,6 @@ struct desc_b200_handle {
     double* S0 = nullptr;       // n_slots
     bool has_dup_apex = false;  // explicit cycle lists that repeat an apex within an edge (CEMP's with-replacement draw)
 
-    // lane-per-edge PGD layout (pgd_ell.cuh): slot arrays of the local vertex blocks re-ordered into tiles of
-    // 32/G edges, slot s of the tile's edge q at tile_base + (s/G)*32 + q*G + s%G, padded with zeros
-    int ell_G = 0;              // lanes per edge (0: layout not built)
-    int ell_ntiles = 0;
-    int64_t ell_size = 0;       // padded slot count
-    int* ell_vtile = nullptr;   // (local vertices + 1): first tile of every local vertex block
-    int4* ell_tiles = nullptr;  // per tile: {base lo, base hi, first edge, steps}
-    int* ell_tcnt = nullptr;    // per tile: edges in the tile
-    bool ell_have_d = false;    // ell_d holds the current S0
-    double* ell_d = nullptr;    // S0
-    uint16_t* ell_rk = nullptr; // rk_i words (rank of the apex in row i | IKJ_appears | JKI_appears)
-    uint32_t* ell_pj = nullptr; // pk_jk words (e_jk | SEL | JKI_appears)
-    double* ell_w[2] = {nullptr, nullptr};
-    double* ell_adam_m = nullptr;
-    double* ell_adam_v = nullptr;
-    bool adam_valid = false;    // the Adam moments on this handle continue a rule with t > 0
-    int adam_layout = 0;        // 0: CSR order (adam_m/adam_v), 1: ELL order (ell_adam_*)
-
     // PGD state -------------------------------------------------------------------------
     double* w[2] = {nullptr, nullptr};     // n_slots each (ping-pong)
     double* S[2] = {nullptr, nullptr};     // m each
@@ -165,6 +147,7 @@ struct desc_b200_handle {
     double* S_adj = nullptr;                // 2m+4 (streamed path): S of the current state in adjacency order
     double* adam_m = nullptr;
     double* adam_v = nullptr;
+    bool adam_valid = false;                // the Adam moments on this handle continue a rule with t > 0
     int final_buf = 0;                      // which ping-pong buffer holds the result
     double* d_hist = nullptr;               // 2*iters
     int hist_cap = 0;
@@ -250,7 +233,7 @@ int desc_allreduce_sum(desc_b200_handle* h, double* buf, int64_t count);
 int desc_allgather_ranges(desc_b200_handle* h, void* buf, size_t elem_bytes,
                           const std::vector<int64_t>& bounds);
 int desc_reduce_to_owners(desc_b200_handle* h, double* buf, int width, const std::vector<int64_t>& bounds,
-                          int tail, bool body_u64 = false);
+                          int tail);
 // Peer-memory exchanges of the PGD iteration (comm.cu): S[0], S[1] and a receive scratch live in a region that every
 // rank maps from every peer (CUDA IPC over NVLink); the exchanges are plain stores into the peers' memory plus a
 // flag barrier.  desc_sym_setup returns DESC_B200_OK with h->sym == nullptr when peer mapping is unavailable or

@@ -1,7 +1,7 @@
 // A6-A12: projected gradient descent over the per-cycle weights (reference: DESC.m:148-261).
 //
-// One fused kernel per iteration.  A group of G lanes owns one edge l=(i,j) and keeps its
-// <= G*EPL slots in registers; for state t-1 -> t it
+// Every iteration takes state t-1 to state t.  A group of G lanes owns one edge l=(i,j) and keeps
+// its <= G*EPL slots in registers; it
 //   * gathers S_{t-1}[e_jk], S_{t-1}[e_ki]                                   (DESC.m:193)
 //   * adds the partner sums A_l, B_l gated by the slot's appears flags        (DESC.m:189-193)
 //   * removes the edge's mean gradient ("Riemannian" projection)              (DESC.m:195-204)
@@ -28,24 +28,27 @@
 // until the active set stops shrinking.  It converges to the same threshold as the reference's
 // sort-and-scan (DESC.m:215-223) without sorting.
 //
-// Two implementations of the iteration share the arithmetic above:
+// Three implementations share the arithmetic above; desc_pgd_impl picks one per solve.
 //
-//  * vertex-blocked (default): edges are (i,j)-sorted, so all edges with the same smaller endpoint
-//    i form one contiguous "vertex block".  One CTA per block keeps in shared memory (a) the S
-//    values of every edge incident to i, indexed by the rank of the other endpoint in i's adjacency
-//    row, and (b) per-warp private partner-sum accumulators with the same indexing.  For a slot
-//    (ij;k) the partner edge {i,k} is then a shared-memory lookup (rank stored per slot as 15 bits
-//    + the IKJ_appears flag); only S[{j,k}] is a global (L2-resident) gather.  The scatter "via i"
-//    is a plain read-modify-write in the warp-private table (apices within one edge are distinct,
-//    one edge per warp instruction => no conflicts), flushed once per CTA.  The scatter "via j"
-//    runs in a second, vertex-centric kernel (k_pgd_scatter<false>) that walks the slot lists of
-//    the edges whose LARGER endpoint is the vertex.  No atomics anywhere: every accumulator entry
-//    is owned by exactly one CTA per kernel, so the result is bit-reproducible, and the random
-//    8-byte traffic of the generic kernel (2 gathers + 2 atomics per slot) drops to one gather.
-//    Streamed bytes per slot: 30 (fused kernel) + 10 (scatter kernel) = the 40 B/slot of SURVEY 8d.
+//  * streamed (default; k_pgd_stream in pgd_stream.cuh, k_pgd_passb in pgd_passb.cuh): two passes per
+//    iteration over per-vertex shared-memory tables.  Edges are (i,j)-sorted, so the edges with the same
+//    smaller endpoint i form one contiguous "vertex block".  For a slot (ij;k) the partner edge {i,k} is
+//    incident to i and {j,k} to j, so every S lookup and partner-sum update is a table operation indexed
+//    by the rank of k in that vertex's adjacency row (rk_i, rk_j: 14 bits + appears flags).  Pass 1 (one
+//    CTA per vertex block, TMA-fed) updates the edges and scatters "via i"; pass 2 (one CTA per vertex v,
+//    in-edges (u,v) with u < v) writes sjk = S_t[e_jk] for the next pass 1 and scatters "via j".  The
+//    scatters are read-modify-writes in warp-private tables (apices within one edge are distinct, one
+//    edge per warp instruction => no conflicts), flushed once per CTA.  No atomics: every partner-sum
+//    entry is owned by exactly one CTA per kernel, so the result is bit-reproducible.
+//  * blocked (k_pgd_block + k_pgd_scatter<false>): the same tables with direct loads and an L2 gather of
+//    S[e_jk].  Taken on single-GPU handles of sparse graphs (m < 100 n, where the streamed kernel's
+//    per-block prologue dominates), and when the streamed passes do not fit (slot lists longer than 256,
+//    or tables too large for their shared memory).
+//  * generic (k_pgd_iter): edge-range kernel with FP64 atomicAdd scatter.  Taken when a vertex degree
+//    exceeds the shared-memory table (DESC_BLOCKED_MAXDEG).
 //
-//  * generic (fallback when a vertex degree exceeds the shared-memory table, or
-//    DESC_B200_PGD_PATH=generic): edge-range kernel with FP64 atomicAdd scatter.
+// DESC_B200_PGD_PATH=stream|blocked|generic forces a path (tests); a forced stream still takes the
+// blocked kernels when the graph does not fit the streamed ones.
 #include "internal.cuh"
 
 #include <algorithm>
@@ -615,7 +618,6 @@ k_pgd_partials(const double* __restrict__ partial, int nblocks, const int* __res
 
 #include "pgd_stream.cuh"
 #include "pgd_passb.cuh"
-#include "pgd_ell.cuh"
 
 template <int G, int EPL, int NCW, int NSW>
 static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, int want_ctas, bool dry) {
@@ -625,31 +627,6 @@ static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, i
     StreamArgs sa;
     sa.b = a;
     sa.max_ns = h->max_ns;
-    sa.trace = nullptr;
-    sa.trace_cta = 0;
-    static long long* g_trace = nullptr;
-    if (const char* tr = getenv("DESC_B200_TRACE")) {
-        if (!g_trace) {
-            cudaMalloc(&g_trace, 64 * 8 * sizeof(long long));
-            cudaMemset(g_trace, 0, 64 * 8 * sizeof(long long));
-        }
-        sa.trace = g_trace;
-        sa.trace_cta = atoi(tr);
-        static int calls = 0;
-        if (++calls == 12) {   // dump the trace of the 11th launch
-            long long hbuf[64 * 8];
-            cudaStreamSynchronize(h->stream);
-            cudaMemcpy(hbuf, g_trace, sizeof(hbuf), cudaMemcpyDeviceToHost);
-            FILE* f = fopen("gpurun_out/trace.txt", "w");
-            if (f) {
-                for (int t = 0; t < 64; t++) {
-                    for (int k = 0; k < 8; k++) fprintf(f, "%lld ", hbuf[t * 8 + k]);
-                    fprintf(f, "\n");
-                }
-                fclose(f);
-            }
-        }
-    }
     sa.tsc = (TE * h->max_ns + G * EPL + 16 + 7) & ~7;
     const size_t fixed = st_fixed_bytes(a.tstride, h->max_ns, NSW), stage = st_stage_bytes(sa.tsc, TE) + st_hdr_bytes(TE);
     // several CTAs per SM: one CTA's table prologue / flush overlaps the others' streaming.
@@ -746,34 +723,7 @@ static int launch_scatter(desc_b200_handle* h, const BlkArgs& a, const double* w
 }
 
 // pass over larger endpoints of the streamed path: sjk <- S_t[e_jk], partner sums "via j" of w_t
-// (DESC_B200_PASSB=tma selects the TMA-fed kernel instead of the register-prefetch one; measured on
-// B200 at cfg 4: 1.58 ms vs 1.12 ms - two small bulk copies per in-edge are issue-bound)
 static int launch_passb(desc_b200_handle* h, const BlkArgs& a, const double* w_t) {
-    const char* mode = getenv("DESC_B200_PASSB");
-    if (mode && strcmp(mode, "tma") == 0) {
-        PassbArgs pa;
-        pa.b = a;
-        pa.w = w_t;
-        pa.jhdr = h->jhdr;
-        pa.sjk = h->sjk;
-        pa.wmax = (h->max_ns + 1 + 1) & ~1;
-        pa.rmax = (h->max_ns + 7 + 7) & ~7;
-        const size_t fixed = pt_fixed_bytes(a.tstride), stage = pt_stage_bytes(pa.wmax, pa.rmax);
-        int nst = 0;
-        for (int ctas = 2; ctas >= 1 && !nst; ctas--) {
-            const size_t budget = (size_t)(228 * 1024) / ctas - 1024 - 256;
-            for (int c = PT_MAXSTAGES; c >= 2 && !nst; c--)
-                if (fixed + c * stage <= budget) nst = c;
-        }
-        if (nst) {
-            pa.nstages = nst;
-            const size_t smem = fixed + nst * stage;
-            CUDA_TRY(cudaFuncSetAttribute(k_pgd_passb_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            k_pgd_passb_tma<<<h->n, PT_TB, smem, h->stream>>>(pa);
-            KERNEL_CHECK(h);
-            return DESC_B200_OK;
-        }
-    }
     // warps per CTA by the mean number of local in-edges per vertex (batches of PB_U edges per warp)
     const double per_cta = (double)(h->e_end - h->e_begin) / std::max(h->n, 1);
     // (2-warp CTAs were used for the small per-vertex work of 4-8 GPU shards; measured on one rank's share of an
@@ -786,8 +736,8 @@ static int launch_passb(desc_b200_handle* h, const BlkArgs& a, const double* w_t
     const size_t smem = (size_t)(2 + nw) * a.tstride * sizeof(double);   // T_S, nw private tables, header tile
 #define PB_LAUNCH(NW)                                                                                              \
     {                                                                                                              \
-        CUDA_TRY(cudaFuncSetAttribute(k_pgd_passb<true, NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_pgd_passb<true, NW><<<h->n, NW * 32, smem, h->stream>>>(a, w_t, h->jhdr, h->sjk, (h->max_ns + 31) / 32);                          \
+        CUDA_TRY(cudaFuncSetAttribute(k_pgd_passb<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));       \
+        k_pgd_passb<NW><<<h->n, NW * 32, smem, h->stream>>>(a, w_t, h->jhdr, h->sjk, (h->max_ns + 31) / 32);           \
     }
     if (nw >= 8) PB_LAUNCH(8) else if (nw >= 4) PB_LAUNCH(4) else PB_LAUNCH(2)
 #undef PB_LAUNCH
@@ -830,108 +780,6 @@ static int launch_iter_any(desc_b200_handle* h, const PgdArgs& a, int rule_kind)
     return DESC_B200_ERR_LIMIT;
 }
 
-// ------------------------------------------------------------------------------------------
-// lane-per-edge path (pgd_ell.cuh): layout construction and launches
-// ------------------------------------------------------------------------------------------
-static int ell_pick_G(int max_ns) {
-    int G = 1;
-    while (G * 32 < max_ns) G <<= 1;
-    return G;
-}
-
-// Tile directory + the iteration-invariant index arrays in ELL order; built once per incidence.
-static int ell_build(desc_b200_handle* h) {
-    if (h->ell_G) return DESC_B200_OK;
-    const int G = ell_pick_G(std::max(h->max_ns, 1));
-    if (G > 32 || !h->rk_i) return DESC_B200_ERR_LIMIT;
-    cudaStream_t st = h->stream;
-    const int TE = 32 / G;
-    const int nv = h->v_end - h->v_begin;
-    std::vector<int> vtile(nv + 1, 0), te0, tcnt;
-    for (int v = h->v_begin; v < h->v_end; v++) {
-        vtile[v - h->v_begin] = (int)te0.size();
-        for (int e = h->h_estart[v]; e < h->h_estart[v + 1]; e += TE) {
-            te0.push_back(e);
-            tcnt.push_back(std::min(TE, h->h_estart[v + 1] - e));
-        }
-    }
-    vtile[nv] = (int)te0.size();
-    const int nt = (int)te0.size();
-    int *d_te0 = nullptr, *d_tcnt = nullptr, *d_sizes = nullptr;
-    int64_t* d_tbase = nullptr;
-    CUDA_TRY(cudaMalloc(&h->ell_vtile, (size_t)(nv + 1) * sizeof(int)));
-    CUDA_TRY(cudaMemcpyAsync(h->ell_vtile, vtile.data(), (size_t)(nv + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMalloc(&d_te0, (size_t)std::max(nt, 1) * sizeof(int)));
-    CUDA_TRY(cudaMalloc(&d_tcnt, (size_t)std::max(nt, 1) * sizeof(int)));
-    CUDA_TRY(cudaMalloc(&d_sizes, (size_t)std::max(nt, 1) * sizeof(int)));
-    CUDA_TRY(cudaMalloc(&d_tbase, (size_t)(nt + 1) * sizeof(int64_t)));
-    CUDA_TRY(cudaMalloc(&h->ell_tiles, (size_t)std::max(nt, 1) * sizeof(int4)));
-    int64_t total = 0;
-    if (nt > 0) {
-        CUDA_TRY(cudaMemcpyAsync(d_te0, te0.data(), (size_t)nt * sizeof(int), cudaMemcpyHostToDevice, st));
-        CUDA_TRY(cudaMemcpyAsync(d_tcnt, tcnt.data(), (size_t)nt * sizeof(int), cudaMemcpyHostToDevice, st));
-        k_ell_steps<<<(nt + 255) / 256, 256, 0, st>>>(d_te0, d_tcnt, nt, h->rowptr, G, d_sizes);
-        KERNEL_CHECK(h);
-        DESC_TRY(desc_exclusive_scan_i64(h, d_sizes, d_tbase, nt));
-        CUDA_TRY(cudaMemcpyAsync(&total, d_tbase + nt, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-        k_ell_tiles<<<(nt + 255) / 256, 256, 0, st>>>(d_te0, d_sizes, d_tbase, nt, h->ell_tiles);
-        KERNEL_CHECK(h);
-        CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    // d_tcnt is kept inside the permutation launches below only; free the rest
-    h->ell_ntiles = nt;
-    h->ell_size = total;
-    const size_t na = (size_t)std::max<int64_t>(total, 1) + 32;
-    CUDA_TRY(cudaMalloc(&h->ell_d, na * sizeof(double)));
-    CUDA_TRY(cudaMalloc(&h->ell_rk, na * sizeof(uint16_t)));
-    CUDA_TRY(cudaMalloc(&h->ell_pj, na * sizeof(uint32_t)));
-    for (int b = 0; b < 2; b++) {
-        CUDA_TRY(cudaMalloc(&h->ell_w[b], na * sizeof(double)));
-        CUDA_TRY(cudaMemsetAsync(h->ell_w[b], 0, na * sizeof(double), st));
-    }
-    if (nt > 0) {
-        k_ell_permute<1><<<DESC_SMS * 8, 256, 0, st>>>(h->ell_tiles, d_tcnt, nt, G, h->rowptr, h->slot_base, h->rk_i, h->pk_jk,
-                                                      nullptr, h->ell_rk, h->ell_pj, nullptr, nullptr, nullptr);
-        KERNEL_CHECK(h);
-    }
-    CUDA_TRY(cudaStreamSynchronize(st));
-    CUDA_TRY(cudaFree(d_te0));
-    CUDA_TRY(cudaFree(d_sizes));
-    CUDA_TRY(cudaFree(d_tbase));
-    h->ell_tcnt = d_tcnt;
-    h->ell_G = G;
-    h->ell_have_d = false;
-    return DESC_B200_OK;
-}
-
-template <int G, int EPL, int RULE, int MODE>
-static int launch_ell_t(desc_b200_handle* h, const EllArgs& ea, int nv) {
-    const size_t smem = ell_smem_bytes(ea.tstride, ea.max_ns);
-    if (smem > 200 * 1024) return DESC_B200_ERR_LIMIT;
-    CUDA_TRY(cudaFuncSetAttribute(k_pgd_ell<G, EPL, RULE, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_pgd_ell<G, EPL, RULE, MODE><<<nv, ELL_TB, smem, h->stream>>>(ea);
-    KERNEL_CHECK(h);
-    return DESC_B200_OK;
-}
-
-template <int RULE, int MODE>
-static int launch_ell(desc_b200_handle* h, const EllArgs& ea) {
-    const int nv = h->v_end - h->v_begin;
-    if (nv <= 0) return DESC_B200_OK;
-    switch (h->ell_G) {
-        case 1:
-            if (h->max_ns <= 8) return launch_ell_t<1, 8, RULE, MODE>(h, ea, nv);
-            if (h->max_ns <= 16) return launch_ell_t<1, 16, RULE, MODE>(h, ea, nv);
-            return launch_ell_t<1, 32, RULE, MODE>(h, ea, nv);
-        case 2: return launch_ell_t<2, 32, RULE, MODE>(h, ea, nv);
-        case 4: return launch_ell_t<4, 32, RULE, MODE>(h, ea, nv);
-        case 8: return launch_ell_t<8, 32, RULE, MODE>(h, ea, nv);
-        case 16: return launch_ell_t<16, 32, RULE, MODE>(h, ea, nv);
-        case 32: return launch_ell_t<32, 32, RULE, MODE>(h, ea, nv);
-    }
-    return DESC_B200_ERR_LIMIT;
-}
-
 // step size of call number t (1-based count of GetStep calls on the rule object)
 static double step_size(const desc_b200_step_rule* r, int64_t t) {
     switch (r->kind) {
@@ -963,188 +811,10 @@ static int exchange_S(desc_b200_handle* h, int which) {
     if (h->sym && h->S_in_sym) return desc_sym_allgather_S(h, which, h->shard_edges);
     return desc_allgather_ranges(h, h->S[which], sizeof(double), h->shard_edges);
 }
-static int exchange_partner_sums(desc_b200_handle* h, int which, bool body_u64) {
+static int exchange_partner_sums(desc_b200_handle* h, int which) {
     if (h->world <= 1) return DESC_B200_OK;
-    if (h->sym && !body_u64) return desc_sym_reduce_to_owners(h, h->acc[which], h->shard_edges);
-    return desc_reduce_to_owners(h, h->acc[which], 2, h->shard_edges, 2, body_u64);
-}
-
-// The lane-per-edge path: state 0, the iterations with the reference's lagged early stop, the objective of the
-// last state; same bookkeeping kernels and history layout as the other paths.
-static int desc_pgd_ell(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int* iters_run) {
-    cudaStream_t st = h->stream;
-    const int64_t m = h->m;
-    const int64_t nacc = 2 * m + 2;
-    const bool adam = rule->kind == 2 && rule->strategy == 0;
-    DESC_TRY(ell_build(h));
-    const int nt = h->ell_ntiles;
-    if (!h->ell_have_d && nt > 0) {
-        k_ell_permute<2><<<DESC_SMS * 8, 256, 0, st>>>(h->ell_tiles, h->ell_tcnt, nt, h->ell_G, h->rowptr, h->slot_base, nullptr,
-                                                      nullptr, h->S0, nullptr, nullptr, h->ell_d, nullptr, nullptr);
-        KERNEL_CHECK(h);
-    }
-    h->ell_have_d = true;
-    if (adam) {
-        const size_t nb = ((size_t)std::max<int64_t>(h->ell_size, 1) + 32) * sizeof(double);
-        const bool fresh = !h->ell_adam_m;
-        if (!h->ell_adam_m) CUDA_TRY(cudaMalloc(&h->ell_adam_m, nb));
-        if (!h->ell_adam_v) CUDA_TRY(cudaMalloc(&h->ell_adam_v, nb));
-        if (rule->t > 0 && (fresh || !h->adam_valid || h->adam_layout != 1)) {
-            desc_set_error("HybridGradient rule with t=%lld > 0, but this handle holds no Adam moments that continue it "
-                           "(new handle, rebuilt incidence, or a run that was stopped early): HybridGradient.m:24-27 "
-                           "zeroes m_t / v_t only at t == 0", (long long)rule->t);
-            return DESC_B200_ERR_STATE;
-        }
-        if (rule->t == 0) {  // HybridGradient.m:24-27: state is zeroed on the first call only
-            CUDA_TRY(cudaMemsetAsync(h->ell_adam_m, 0, nb, st));
-            CUDA_TRY(cudaMemsetAsync(h->ell_adam_v, 0, nb, st));
-        }
-        h->adam_layout = 1;
-        h->adam_valid = false;   // becomes valid again when this run ends without an early stop
-    }
-    const int nv = h->v_end - h->v_begin;
-    EllArgs ea;
-    PgdArgs& a = ea.p;
-    a.rowptr = h->rowptr;
-    a.pk_jk = nullptr;
-    a.pk_ki = nullptr;
-    a.S0 = nullptr;
-    a.adam_m = h->ell_adam_m;
-    a.adam_v = h->ell_adam_v;
-    a.ctrl = h->d_ctrl;
-    a.e0 = h->e_begin;
-    a.e1 = h->e_end;
-    a.slot_base = h->slot_base;
-    a.m = m;
-    a.beta1 = rule->beta_1;
-    a.beta2 = rule->beta_2;
-    a.corr1 = a.corr2 = 1.0;
-    a.lr = 0.0;
-    ea.tiles = h->ell_tiles;
-    ea.vtile = h->ell_vtile;
-    ea.d = h->ell_d;
-    ea.rk = h->ell_rk;
-    ea.pj = h->ell_pj;
-    ea.rowstart = h->rowstart;
-    ea.adj_nbr = h->adj_nbr;
-    ea.adj_eid = h->adj_eid;
-    ea.estart = h->estart;
-    ea.v0 = h->v_begin;
-    ea.tstride = (h->maxdeg + 1 + 3) & ~3;
-    ea.max_ns = std::max(h->max_ns, 1);
-    ea.partial = h->pgd_partial;
-    const int launches0 = h->launches;
-
-    // ---- state 0 (DESC.m:148-157)
-    CUDA_TRY(cudaMemsetAsync(h->acc[0], 0, nacc * sizeof(double), st));
-    a.w_cur = nullptr;
-    a.w_next = h->ell_w[0];
-    a.S_cur = nullptr;
-    a.S_next = h->S[0];
-    a.acc_cur = nullptr;
-    a.acc_next = h->acc[0];
-    if (nt > 0) DESC_TRY((launch_ell<0, 1>(h, ea)));
-    DESC_TRY(exchange_S(h, 0));
-    DESC_TRY(exchange_partner_sums(h, 0, true));
-
-    std::vector<cudaEvent_t>& evs = h->iter_events;
-    while ((int)evs.size() < 5 * std::min(iters, 512)) {
-        cudaEvent_t e;
-        CUDA_TRY(cudaEventCreate(&e));
-        evs.push_back(e);
-    }
-    int t_done = 0;
-    bool stopped = false;
-    const int check_every = h->diag_on ? 1 : 8;
-    for (int t = 1; t <= iters && !stopped; t++) {
-        const int cur = (t - 1) & 1, nxt = t & 1;
-        CUDA_TRY(cudaMemsetAsync(h->acc[nxt], 0, nacc * sizeof(double), st));
-        a.w_cur = h->ell_w[cur];
-        a.w_next = h->ell_w[nxt];
-        a.S_cur = h->S[cur];
-        a.S_next = h->S[nxt];
-        a.acc_cur = h->acc[cur];
-        a.acc_next = h->acc[nxt];
-        const int64_t tcall = rule->t + t;
-        a.lr = step_size(rule, tcall);
-        if (adam) {
-            a.corr1 = 1.0 - std::pow(rule->beta_1, (double)tcall);
-            a.corr2 = 1.0 - std::pow(rule->beta_2, (double)tcall);
-        }
-        const bool timed = t <= 512;
-        if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1)], st));
-        if (nt > 0) {
-            if (adam)
-                DESC_TRY((launch_ell<1, 0>(h, ea)));
-            else
-                DESC_TRY((launch_ell<0, 0>(h, ea)));
-        }
-        if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 1], st));
-        k_pgd_partials<<<1, PGD_PART_TB, 0, st>>>(h->pgd_partial, nt > 0 ? nv : 0, h->d_ctrl, h->acc[nxt] + 2 * m);
-        KERNEL_CHECK(h);
-        if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 3], st));
-        DESC_TRY(exchange_S(h, nxt));
-        DESC_TRY(exchange_partner_sums(h, nxt, true));
-        if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 4], st));
-        if (h->diag_on) DESC_TRY(desc_diag_record(h, t, h->S[nxt]));
-        k_pgd_finalize<<<1, 1, 0, st>>>(h->acc[nxt] + 2 * m, t, 0, m, 1e-5, 30, h->d_hist, h->d_ctrl, h->d_ctrl_f);
-        KERNEL_CHECK(h);
-        t_done = t;
-        if (t % check_every == 0 || t == iters) {
-            CUDA_TRY(cudaMemcpyAsync(h->h_ctrl, h->d_ctrl, 4 * sizeof(int), cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(cudaStreamSynchronize(st));
-            stopped = h->h_ctrl[0] != 0;
-        }
-    }
-    int final_iter = 0;
-    if (stopped) {
-        final_iter = h->h_ctrl[1];
-    } else if (iters > 0) {
-        const int cur = iters & 1, nxt = (iters + 1) & 1;
-        CUDA_TRY(cudaMemsetAsync(h->acc[nxt] + 2 * m, 0, 2 * sizeof(double), st));
-        a.w_cur = h->ell_w[cur];
-        a.S_cur = h->S[cur];
-        a.acc_cur = h->acc[cur];
-        a.acc_next = h->acc[nxt];
-        if (nt > 0) DESC_TRY((launch_ell<0, 2>(h, ea)));
-        k_pgd_partials<<<1, PGD_PART_TB, 0, st>>>(h->pgd_partial, nt > 0 ? nv : 0, h->d_ctrl, h->acc[nxt] + 2 * m);
-        KERNEL_CHECK(h);
-        if (h->world > 1) DESC_TRY(desc_allreduce_sum(h, h->acc[nxt] + 2 * m, 2));
-        k_pgd_finalize<<<1, 1, 0, st>>>(h->acc[nxt] + 2 * m, iters, 1, m, 1e-5, 30, h->d_hist, h->d_ctrl, h->d_ctrl_f);
-        KERNEL_CHECK(h);
-        final_iter = iters;
-    }
-    // the weights of the final state back in the reference's slot order (getters, later stages)
-    if (nt > 0) {
-        k_ell_permute<4><<<DESC_SMS * 8, 256, 0, st>>>(h->ell_tiles, h->ell_tcnt, nt, h->ell_G, h->rowptr, h->slot_base, nullptr,
-                                                      nullptr, nullptr, nullptr, nullptr, nullptr, h->ell_w[final_iter & 1],
-                                                      h->w[final_iter & 1]);
-        KERNEL_CHECK(h);
-    }
-    CUDA_TRY(cudaStreamSynchronize(st));
-    h->final_buf = final_iter & 1;
-    h->have_pgd = true;
-    *iters_run = final_iter;
-    rule->t += final_iter;
-    if (adam) h->adam_valid = !stopped;   // a stopped run has advanced the moments one launch past the reported state
-    double s1 = 0.0, sc = 0.0;
-    int cnt = 0;
-    for (int t = 1; t <= std::min(std::min(t_done, 512), std::max(final_iter, 1)); t++) {
-        float a1 = 0.f, ar = 0.f;
-        cudaEvent_t* e = &evs[5 * (t - 1)];
-        if (cudaEventElapsedTime(&a1, e[0], e[1]) == cudaSuccess && cudaEventElapsedTime(&ar, e[3], e[4]) == cudaSuccess) {
-            s1 += a1;
-            sc += ar;
-            cnt++;
-        }
-    }
-    DESC_TRY(check_peer_barrier(h));
-    h->tm.pgd_pass1_ms = cnt > 0 ? s1 / cnt : 0.0;
-    h->tm.pgd_pass2_ms = 0.0;
-    h->tm.pgd_comm_ms = cnt > 0 ? sc / cnt : 0.0;
-    h->tm.pgd_iter_ms = h->tm.pgd_pass1_ms;
-    h->tm.pgd_launches = h->launches - launches0;
-    return DESC_B200_OK;
+    if (h->sym) return desc_sym_reduce_to_owners(h, h->acc[which], h->shard_edges);
+    return desc_reduce_to_owners(h, h->acc[which], 2, h->shard_edges, 2);
 }
 
 int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int* iters_run) {
@@ -1201,20 +871,12 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         CUDA_TRY(cudaMalloc(&h->d_hist, (size_t)2 * (iters + 1) * sizeof(double)));
         h->hist_cap = iters + 1;
     }
-    // DESC_B200_PGD_PATH = stream (default) | ell | blocked | generic
-    bool use_ell = false;
-    {
-        const char* force = getenv("DESC_B200_PGD_PATH");
-        const bool want_ell = force && strcmp(force, "ell") == 0;
-        use_ell = want_ell && blocked && ell_pick_G(std::max(h->max_ns, 1)) <= 32 &&
-                  ell_smem_bytes((h->maxdeg + 1 + 3) & ~3, std::max(h->max_ns, 1)) <= 200 * 1024;
-    }
-    if (adam && !use_ell) {
+    if (adam) {
         const size_t nb = (size_t)std::max<int64_t>(h->n_slots, 1) * sizeof(double);
         const bool fresh = !h->adam_m;
         if (!h->adam_m) CUDA_TRY(cudaMalloc(&h->adam_m, nb));
         if (!h->adam_v) CUDA_TRY(cudaMalloc(&h->adam_v, nb));
-        if (rule->t > 0 && (fresh || !h->adam_valid || h->adam_layout != 0)) {
+        if (rule->t > 0 && (fresh || !h->adam_valid)) {
             desc_set_error("HybridGradient rule with t=%lld > 0, but this handle holds no Adam moments that continue it "
                            "(new handle, rebuilt incidence, or a run that was stopped early): HybridGradient.m:24-27 "
                            "zeroes m_t / v_t only at t == 0", (long long)rule->t);
@@ -1224,7 +886,6 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
             CUDA_TRY(cudaMemsetAsync(h->adam_m, 0, nb, st));
             CUDA_TRY(cudaMemsetAsync(h->adam_v, 0, nb, st));
         }
-        h->adam_layout = 0;
         h->adam_valid = false;
     }
     CUDA_TRY(cudaMemsetAsync(h->d_ctrl, 0, 4 * sizeof(int), st));
@@ -1240,7 +901,6 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         // buffers before the fills above have run (a faster peer's slice would be overwritten with ones)
         if (h->S_in_sym) DESC_TRY(desc_sym_barrier(h));
     }
-    if (use_ell) return desc_pgd_ell(h, iters, rule, iters_run);
     PgdArgs a;
     a.rowptr = h->rowptr;
     a.pk_jk = h->pk_jk;
@@ -1323,7 +983,7 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         ba.acc2_next = use_acc2 ? h->acc2[0] : nullptr;
         DESC_TRY(launch_passb(h, ba, h->w[0]));
     }
-    DESC_TRY(exchange_partner_sums(h, 0, false));
+    DESC_TRY(exchange_partner_sums(h, 0));
 
     // per-iteration kernel timing: events around the iteration kernels only
     std::vector<cudaEvent_t>& evs = h->iter_events;
@@ -1391,7 +1051,7 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         }
         if (h->world > 1) {
             // a rank reads only the partner sums of its own edges: deliver each range's sum to its owner
-            DESC_TRY(exchange_partner_sums(h, nxt, false));
+            DESC_TRY(exchange_partner_sums(h, nxt));
             if (!stream) DESC_TRY(exchange_S(h, nxt));
         }
         if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 4], st));

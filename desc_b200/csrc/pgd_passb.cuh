@@ -39,7 +39,7 @@ __device__ __forceinline__ void pb_zero_row(const BlkArgs& a, int v, int rs, int
 // PB_WARPS warps (= private tables) per CTA: 8 when a vertex has hundreds of local in-edges, fewer
 // (smaller CTAs, more of them per SM) when sharding over GPUs leaves each CTA little work, so that
 // the O(degree) table prologue / flush of one CTA overlaps the others'.
-template <bool WRITE_SJK, int PB_WARPS>
+template <int PB_WARPS>
 __global__ void __launch_bounds__(PB_WARPS * 32)
 k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jhdr, double* __restrict__ sjk,
             int cpe) {
@@ -74,7 +74,7 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
 #pragma unroll
         for (int k = 0; k < KU; k++) {
             const int r = rb + k * PB_TB;
-            sv[k] = (WRITE_SJK && r < deg) ? a.S_adj[rs + r] : 0.0;
+            sv[k] = r < deg ? a.S_adj[rs + r] : 0.0;
             hv[k] = lo + r < hi ? __ldg(jhdr + lo + r) : make_int2(0, 0);
         }
 #pragma unroll
@@ -149,9 +149,7 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
         for (int u = 0; u < U; u++) ts[u] = T_S[lane < B.h[u].y ? (B.r[u] & RK_MASK) : dummy];
 #pragma unroll
         for (int u = 0; u < U; u++) {
-            if (WRITE_SJK) {
-                if (lane < B.h[u].y) __stcs(sjk + B.h[u].x + lane, ts[u]);
-            }
+            if (lane < B.h[u].y) __stcs(sjk + B.h[u].x + lane, ts[u]);
             const bool f = (B.r[u] & RK_APP) != 0u;
             const uint32_t ia = f ? (B.r[u] & RK_MASK) : dummy;
             const double t = TA[ia];
@@ -209,180 +207,3 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
     }
 }
 
-
-// ------------------------------------------------------------------------------------------
-// TMA-fed variant (default): the (w, rank) chunks of the in-edges are scattered in memory (one
-// ~240-byte piece per edge), so the direct-load version above is bound by memory latency times its
-// register prefetch depth.  Here a producer warp issues two small cp.async.bulk copies per in-edge
-// (lane = edge, 32 edges per tile) into a ring of shared-memory tiles; mbarriers hand tiles to the
-// scatter warps (one private partner-sum table each) and back.  Bulk copies need 16-byte alignment:
-// each edge's pieces are widened to 16-byte boundaries and land in fixed-size per-edge regions.
-#define PT_NSW 4                        // scatter warps
-#define PT_TB ((PT_NSW + 1) * 32)
-#define PT_TE 32                        // in-edges per tile (one per producer lane)
-#define PT_MAXSTAGES 6
-
-struct PassbArgs {
-    BlkArgs b;
-    const double* w;
-    const int2* jhdr;
-    double* sjk;
-    int wmax;      // doubles per edge region  (multiple of 2)
-    int rmax;      // ranks per edge region    (multiple of 8)
-    int nstages;
-};
-__host__ __device__ __forceinline__ size_t pt_stage_bytes(int wmax, int rmax) {
-    return (size_t)PT_TE * ((size_t)wmax * 8 + (size_t)rmax * 2 + sizeof(int4));
-}
-__host__ __device__ __forceinline__ size_t pt_fixed_bytes(int tstride) {
-    return 128 + (size_t)(1 + PT_NSW) * tstride * sizeof(double);
-}
-
-__global__ void __launch_bounds__(PT_TB)
-k_pgd_passb_tma(PassbArgs pa) {
-    const BlkArgs& a = pa.b;
-    if (a.p.ctrl[0]) return;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw);
-    uint64_t* empty = full + PT_MAXSTAGES;
-    double* T_S = reinterpret_cast<double*>(smem_raw + 128);
-    double* T_acc = T_S + a.tstride;
-    unsigned char* stage0 = reinterpret_cast<unsigned char*>(T_acc + (size_t)PT_NSW * a.tstride);
-    const int wmax = pa.wmax, rmax = pa.rmax, NST = pa.nstages;
-    const size_t off_rk = (size_t)PT_TE * wmax * 8, off_hdr = off_rk + (size_t)PT_TE * rmax * 2;
-    const size_t stage_bytes = pt_stage_bytes(wmax, rmax);
-
-    const int v = (int)gridDim.x - 1 - (int)blockIdx.x;   // long in-edge lists first
-    const int rs = a.rowstart[v];
-    const int deg = a.rowstart[v + 1] - rs;
-    const int ub = min(a.v1, v);                           // neighbours u with v0 <= u < ub
-    if (ub <= a.v0) {
-        pb_zero_row(a, v, rs, deg);
-        return;
-    }
-    const int lo = rs + (a.v0 > 0 ? desc_rank(a.bm, a.bmprefix, a.nwords, v, a.v0) : 0);
-    const int hi = rs + desc_rank(a.bm, a.bmprefix, a.nwords, v, ub);
-    if (hi <= lo) {
-        pb_zero_row(a, v, rs, deg);
-        return;
-    }
-    const int ntiles = (hi - lo + PT_TE - 1) / PT_TE;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NST; s++) {
-            mbar_init(&full[s], 1);
-            mbar_init(&empty[s], PT_NSW);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (warp == PT_NSW) {
-        // ------------------------------------------------------------------ producer (lane = in-edge)
-        const uint64_t pol = l2_evict_first_policy();
-        int s = 0;
-        uint32_t ph = 0;
-        int2 hnext = make_int2(0, 0);
-        if (lo + lane < hi) hnext = __ldg(pa.jhdr + lo + lane);
-        for (int t = 0; t < ntiles; t++) {
-            const int2 h = hnext;
-            const int pn = lo + (t + 1) * PT_TE + lane;
-            hnext = make_int2(0, 0);
-            if (pn < hi) hnext = __ldg(pa.jhdr + pn);      // next tile's headers fly during this tile
-            unsigned char* st = stage0 + (size_t)s * stage_bytes;
-            const int s0 = h.x, ns = h.y;
-            const int wa = s0 & ~1, wcnt = ns > 0 ? ((s0 + ns + 1) & ~1) - wa : 0;
-            const int ra = s0 & ~7, rcnt = ns > 0 ? ((s0 + ns + 7) & ~7) - ra : 0;
-            uint32_t bytes = (uint32_t)(wcnt * 8 + rcnt * 2);
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) bytes += __shfl_xor_sync(0xffffffffu, bytes, o);
-            if (lane == 0) mbar_wait(&empty[s], ph ^ 1u);
-            __syncwarp();
-            reinterpret_cast<int4*>(st + off_hdr)[lane] = make_int4(s0, ns, s0 - wa, s0 - ra);
-            __syncwarp();
-            if (lane == 0) mbar_expect_tx(&full[s], bytes);
-            __syncwarp();
-            if (ns > 0) {
-                bulk_g2s(st + (size_t)lane * wmax * 8, pa.w + wa, (uint32_t)(wcnt * 8), &full[s], pol);
-                bulk_g2s(st + off_rk + (size_t)lane * rmax * 2, a.rk_j + ra, (uint32_t)(rcnt * 2), &full[s], pol);
-            }
-            if (++s == NST) {
-                s = 0;
-                ph ^= 1u;
-            }
-        }
-    } else {
-        // ------------------------------------------------------------------ scatter warps
-        constexpr int NT = PT_NSW * 32;
-        for (int r = threadIdx.x; r < deg; r += NT) {
-            T_S[r] = a.S_adj[rs + r];
-#pragma unroll
-            for (int q = 0; q < PT_NSW; q++) T_acc[q * a.tstride + r] = 0.0;
-        }
-        asm volatile("bar.sync 1, %0;" ::"n"(NT) : "memory");
-        double* TA = T_acc + (size_t)warp * a.tstride;
-        const uint32_t dummy = (uint32_t)a.tstride - 1u;
-        int s = 0;
-        uint32_t ph = 0;
-        for (int t = 0; t < ntiles; t++) {
-            const unsigned char* st = stage0 + (size_t)s * stage_bytes;
-            const int4* hdr = reinterpret_cast<const int4*>(st + off_hdr);
-            mbar_wait(&full[s], ph);
-            constexpr int U = 4;                                   // edges per batch: loads of a batch issue together
-            for (int qb = warp * U; qb < PT_TE; qb += PT_NSW * U) {
-                int4 h4[U];
-                double wv[U], ts[U];
-                uint32_t rk[U];
-#pragma unroll
-                for (int u = 0; u < U; u++) {
-                    h4[u] = hdr[qb + u];
-                    const double* sw = reinterpret_cast<const double*>(st) + (size_t)(qb + u) * wmax + h4[u].z;
-                    const uint16_t* sr = reinterpret_cast<const uint16_t*>(st + off_rk) + (size_t)(qb + u) * rmax + h4[u].w;
-                    const bool ok = lane < h4[u].y;
-                    wv[u] = ok ? sw[lane] : 0.0;
-                    rk[u] = ok ? (uint32_t)sr[lane] : 0u;
-                }
-#pragma unroll
-                for (int u = 0; u < U; u++) ts[u] = T_S[lane < h4[u].y ? (rk[u] & RK_MASK) : dummy];
-#pragma unroll
-                for (int u = 0; u < U; u++) {
-                    if (lane < h4[u].y) __stcs(pa.sjk + h4[u].x + lane, ts[u]);
-                    const bool f = (rk[u] & RK_APP) != 0u;
-                    const uint32_t ia = f ? (rk[u] & RK_MASK) : dummy;
-                    const double tv = TA[ia];
-                    TA[ia] = tv + (f ? wv[u] : 0.0);
-                    __syncwarp();
-                }
-#pragma unroll
-                for (int u = 0; u < U; u++) {
-                    if (h4[u].y > 32) {   // slot lists longer than a warp (ranks of one edge are distinct)
-                        const double* sw = reinterpret_cast<const double*>(st) + (size_t)(qb + u) * wmax + h4[u].z;
-                        const uint16_t* sr = reinterpret_cast<const uint16_t*>(st + off_rk) + (size_t)(qb + u) * rmax + h4[u].w;
-                        for (int i2 = lane + 32; i2 < h4[u].y; i2 += 32) {
-                            const uint32_t rr = sr[i2];
-                            pa.sjk[h4[u].x + i2] = T_S[rr & RK_MASK];
-                            if (rr & RK_APP) TA[rr & RK_MASK] += sw[i2];
-                        }
-                        __syncwarp();
-                    }
-                }
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty[s]);
-            if (++s == NST) {
-                s = 0;
-                ph ^= 1u;
-            }
-        }
-    }
-    __syncthreads();
-    for (int r = threadIdx.x; r < deg; r += PT_TB) {
-        double x = 0.0;
-#pragma unroll
-        for (int q = 0; q < PT_NSW; q++) x += T_acc[q * a.tstride + r];
-        const int64_t pos = pb_acc_pos(a, v, rs, r);   // owned by this CTA within this kernel
-        if (a.acc2_next)
-            a.acc2_next[pos] = x;
-        else
-            a.p.acc_next[pos] += x;
-    }
-}

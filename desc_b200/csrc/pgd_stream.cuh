@@ -33,9 +33,6 @@
 #ifndef ST_PFT
 #define ST_PFT 2                       // L2 prefetch distance of the producer, in tiles (2: 1.29 ms, 3: 1.30, 5: 1.32, 8: 1.37)
 #endif
-#ifndef ST_TPW
-#define ST_TPW 1                       // private partner-sum tables per scatter warp (1 or 2)
-#endif
 
 __device__ __forceinline__ uint32_t st_smem(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -98,11 +95,7 @@ struct StreamArgs {
     const double* sjk;  // S[e_jk] per slot for the current state (pgd_passb.cuh)
     const double* S_adj;    // S_cur in adjacency order (2m + 4: 16-byte widened bulk copy)
     const double* acc2_cur; // partner sums of the pass over larger endpoints (2m), null on multi-GPU handles
-    long long* trace; // DESC_B200_TRACE: per-tile event clocks of one CTA (null = off)
-    int trace_cta;
 };
-#define ST_TRACE(k, t) \
-    do { if (sa.trace && (int)blockIdx.x == sa.trace_cta && (t) < 64 && lane == 0) sa.trace[(t) * 8 + (k)] = clock64(); } while (0)
 
 // shared-memory carve-up: barriers | edge headers[nstages][TE] | 1/c table | T_S[tstride+2] | T_acc[NSW] | stages.
 // One stage: w[tsc] f64 | S0[tsc] f64 | sjk[tsc] f64 | rk_i[tsc] u16 | rowptr[TE+2] i64 |
@@ -115,7 +108,7 @@ __host__ __device__ __forceinline__ size_t st_hdr_bytes(int te) { return (size_t
 __host__ __device__ __forceinline__ size_t st_rcp_bytes(int max_ns) { return ((size_t)(max_ns + 1) * 8 + 15) & ~(size_t)15; }
 __host__ __device__ __forceinline__ size_t st_fixed_bytes(int tstride, int max_ns, int nsw) {
     return 128 + st_rcp_bytes(max_ns) +
-           (size_t)(1 + ST_TPW * nsw) * tstride * sizeof(double) + 16;   // T_S (+2: widened copy) + the scatter warps' private tables
+           (size_t)(1 + nsw) * tstride * sizeof(double) + 16;   // T_S (+2: widened copy) + the scatter warps' private tables
 }
 
 // G lanes per edge with EPL slots each, NCW compute warps, ST_NSW scatter warps (private tables),
@@ -137,8 +130,7 @@ k_pgd_stream(StreamArgs sa) {
     double* rcp = reinterpret_cast<double*>(smem_raw + 128 + (size_t)sa.nstages * st_hdr_bytes(TE));
     double* T_S0 = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(rcp) + st_rcp_bytes(sa.max_ns));
     double* T_acc = T_S0 + a.tstride + 2;
-    constexpr int NTAB = ST_TPW * ST_NSW;
-    unsigned char* stage0 = reinterpret_cast<unsigned char*>(T_acc + (size_t)NTAB * a.tstride);
+    unsigned char* stage0 = reinterpret_cast<unsigned char*>(T_acc + (size_t)ST_NSW * a.tstride);
     const int tsc = sa.tsc;
     const size_t stage_bytes = st_stage_bytes(tsc, TE);
     const size_t off_d = (size_t)tsc * 8, off_sj = (size_t)tsc * 16, off_rk = (size_t)tsc * 24;
@@ -178,7 +170,6 @@ k_pgd_stream(StreamArgs sa) {
     __syncthreads();
 
     double objp = 0.0, chgp = 0.0;
-    if (warp == 0) ST_TRACE(6, 0);
     if (warp == NCW + ST_NSW) {
         // ------------------------------------------------------------------ producer
         // lanes prefetch the slot boundaries of 32 tiles at a time; lane 0 issues the bulk copies
@@ -220,9 +211,7 @@ k_pgd_stream(StreamArgs sa) {
                     const int64_t base = sA & ~(int64_t)7;
                     const int64_t cnt = ((sB + 7) & ~(int64_t)7) - base;
                     unsigned char* st = stage0 + (size_t)s * stage_bytes;
-                    ST_TRACE(0, t);
                     mbar_wait(&empty[s], ph ^ 1u);
-                    ST_TRACE(1, t);
                     mbar_expect_tx(&full[s], (uint32_t)(cnt * 26 + rp_cnt * 8 + (e1 - e0) * (sa.acc2_cur ? 32 : 16) + so_cnt * 8));
                     bulk_g2s_plain(st + off_rp, a.p.rowptr + e0a, (uint32_t)(rp_cnt * 8), &full[s]);
                     bulk_g2s_plain(st + off_acc, a.p.acc_cur + 2 * (int64_t)e0, (uint32_t)((e1 - e0) * 16), &full[s]);
@@ -249,7 +238,7 @@ k_pgd_stream(StreamArgs sa) {
         for (int c = threadIdx.x; c <= sa.max_ns; c += NT) rcp[c] = c > 0 ? 1.0 / (double)c : 0.0;
         for (int r = threadIdx.x; r < deg; r += NT) {
 #pragma unroll
-            for (int q = 0; q < NTAB; q++) T_acc[q * a.tstride + r] = 0.0;
+            for (int q = 0; q < ST_NSW; q++) T_acc[q * a.tstride + r] = 0.0;
         }
         asm volatile("bar.sync 1, %0;" ::"n"(NT) : "memory");
         if (warp < NCW) {
@@ -273,7 +262,6 @@ k_pgd_stream(StreamArgs sa) {
             for (int t = 0; t < ntiles; t++, e += TE) {
                 const int64_t* rp = reinterpret_cast<const int64_t*>(st + off_rp) + eoff;
                 mbar_wait(&full[s], ph);
-                if (warp == 0) ST_TRACE(2, t);
                 int sl = 0, ns = 0;
                 int64_t s0 = 0;
                 double A = 0.0, B = 0.0, Sold = 0.0;
@@ -390,7 +378,6 @@ k_pgd_stream(StreamArgs sa) {
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // w_t tile: generic writes -> bulk store
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&done[s]);
-                if (warp == 0) ST_TRACE(3, t);
                 st += stage_bytes;
                 if (++s == NST) {
                     s = 0;
@@ -401,7 +388,7 @@ k_pgd_stream(StreamArgs sa) {
         } else {
             // -------------------------------------------------------------- scatter
             const int swi = warp - NCW;
-            double* Tw = T_acc + (size_t)(ST_TPW * swi) * a.tstride;
+            double* Tw = T_acc + (size_t)swi * a.tstride;
             const uint32_t dummy = (uint32_t)a.tstride - 1u;
             const uint64_t pol = l2_evict_first_policy();
             int s = 0;
@@ -412,7 +399,6 @@ k_pgd_stream(StreamArgs sa) {
                 const uint16_t* srk = reinterpret_cast<const uint16_t*>(st + off_rk);
                 const int64_t* rp = reinterpret_cast<const int64_t*>(st + off_rp) + eoff;
                 mbar_wait(&done[s], ph);
-                if (swi == 0) ST_TRACE(4, t);
                 if (swi == 0 && lane < 3) {
                     // w_t tile -> global: 16-byte aligned interior as one bulk store, ragged ends directly
                     const int e0 = e_lo + t * TE, e1 = min(e0 + TE, e_hi);
@@ -428,9 +414,9 @@ k_pgd_stream(StreamArgs sa) {
                         if (iB < sB && sB - 1 >= iA) a.p.w_next[sB - 1] = sw[sB - 1 - base];
                     }
                 }
-                // This warp's edges q = swi, swi + NSW, ... in batches of U; even / odd edges of a batch go
-                // to the warp's two private tables, so two read-modify-write chains are in flight, and the
-                // (w, rank) loads of the next batch are issued before the current batch's chains.
+                // This warp's edges q = swi, swi + NSW, ... in batches of U, one edge after the other into the
+                // warp's private table; the (w, rank) loads of the next batch are issued before the current
+                // batch's read-modify-writes.
                 constexpr int U = 4;
                 constexpr int NK = (TE + ST_NSW - 1) / ST_NSW;      // edges per scatter warp and tile
                 constexpr int NB = (NK + U - 1) / U;
@@ -457,35 +443,21 @@ k_pgd_stream(StreamArgs sa) {
                 for (int b = 0; b < NB; b++) {
                     if (b + 1 < NB) load_batch(b + 1, nsn, offn, wn, rn);
 #pragma unroll
-                    for (int u = 0; u < U; u += 2) {
-                        double* TA = Tw;
-                        double* TB = Tw + (ST_TPW - 1) * a.tstride;
+                    for (int u = 0; u < U; u++) {
                         // branch-free: lanes without the flag update the dummy entry with 0
-                        const bool fa = (rk[u] & RK_APP) != 0u, fb = (rk[u + 1] & RK_APP) != 0u;
-                        const uint32_t ia = fa ? (rk[u] & RK_MASK) : dummy, ib = fb ? (rk[u + 1] & RK_MASK) : dummy;
-                        if (ST_TPW == 2) {   // two independent chains in flight
-                            const double ta = TA[ia];
-                            const double tb = TB[ib];
-                            TA[ia] = ta + (fa ? wv[u] : 0.0);
-                            TB[ib] = tb + (fb ? wv[u + 1] : 0.0);
-                            __syncwarp();
-                        } else {             // one table: edge after edge
-                            const double ta = TA[ia];
-                            TA[ia] = ta + (fa ? wv[u] : 0.0);
-                            __syncwarp();
-                            const double tb = TA[ib];
-                            TA[ib] = tb + (fb ? wv[u + 1] : 0.0);
-                            __syncwarp();
-                        }
+                        const bool f = (rk[u] & RK_APP) != 0u;
+                        const uint32_t ia = f ? (rk[u] & RK_MASK) : dummy;
+                        const double x = Tw[ia];
+                        Tw[ia] = x + (f ? wv[u] : 0.0);
+                        __syncwarp();
                     }
                     // slot lists longer than a warp (ranks of one edge are distinct: no ordering needed inside)
 #pragma unroll
                     for (int u = 0; u < U; u++) {
                         if (nsu[u] > 32) {
-                            double* TT = Tw + (u & (ST_TPW - 1)) * a.tstride;
                             for (int i2 = lane + 32; i2 < nsu[u]; i2 += 32) {
                                 const uint32_t rr = srk[offu[u] + i2];
-                                if (rr & RK_APP) TT[rr & RK_MASK] += sw[offu[u] + i2];
+                                if (rr & RK_APP) Tw[rr & RK_MASK] += sw[offu[u] + i2];
                             }
                             __syncwarp();
                         }
@@ -498,11 +470,9 @@ k_pgd_stream(StreamArgs sa) {
                         rk[u] = rn[u];
                     }
                 }
-                if (swi == 0) ST_TRACE(7, t);
                 if (swi == 0 && lane == 0) bulk_wait_read0();   // the bulk store has read the stage
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&empty[s]);
-                if (swi == 0) ST_TRACE(5, t);
                 st += stage_bytes;
                 if (++s == NST) {
                     s = 0;
@@ -514,7 +484,6 @@ k_pgd_stream(StreamArgs sa) {
         }
     }
     __syncthreads();
-    if (warp == 0) ST_TRACE(6, 1);
     // flush the private tables: every (edge, side) entry belongs to exactly one vertex block, and this
     // kernel is the first writer of acc_next in an iteration => plain stores (the pass over larger
     // endpoints stores its share into acc2_next, or adds it here on multi-GPU handles)
@@ -534,7 +503,7 @@ k_pgd_stream(StreamArgs sa) {
                 if (r < deg) {
                     double x = 0.0;
 #pragma unroll
-                    for (int q = 0; q < NTAB; q++) x += T_acc[q * a.tstride + r];
+                    for (int q = 0; q < ST_NSW; q++) x += T_acc[q * a.tstride + r];
                     a.p.acc_next[pos[k]] = x;
                 }
             }
@@ -558,5 +527,4 @@ k_pgd_stream(StreamArgs sa) {
         a.partial[2 * blockIdx.x] = o;
         a.partial[2 * blockIdx.x + 1] = c;
     }
-    if (warp == 0) ST_TRACE(6, 2);
 }

@@ -66,11 +66,8 @@ def _check(Ind, RijMat, rule_c, rule_o, iters, ns, seed=3):
     return c
 
 
-@pytest.mark.parametrize("passb", ["direct", "tma"])
 @pytest.mark.parametrize("ns", [32, 33, 64, 65])
-def test_rows_without_lower_or_upper_neighbours(monkeypatch, passb, ns):
-    if passb == "tma":
-        monkeypatch.setenv("DESC_B200_PASSB", "tma")
+def test_rows_without_lower_or_upper_neighbours(ns):
     Ind, RijMat = _holes_graph()
     deg = _degrees(Ind, 200)
     assert np.any(np.cumsum(deg)[:-1] % 2 == 1)               # odd row offsets: the widened S-table copy
