@@ -74,8 +74,8 @@ void desc_b200_destroy(desc_b200_handle* h) {
                     h->d_ctrl_f, h->omega, h->isd, h->X[0], h->X[1], h->gcw_coef, h->gcw_red,
                     h->gcw_small, h->gcw_res, h->R_est, h->d_err, h->d_Sin, h->rk_i, h->rk_j, h->estart,
                     h->pgd_partial, h->jhdr, h->sjk, h->thr_key, h->thr_k, h->comm_scratch,
-                    h->cemp_S[0], h->cemp_S[1], h->diag_work, h->diag_hist, h->R_mst, h->gcw_coef_adj, h->acc2[0],
-                    h->acc2[1], h->S_adj};
+                    h->cemp_S[0], h->cemp_S[1], h->diag_work, h->diag_hist, h->R_mst, h->gcw_coef_adj, h->P1,
+                    h->S_adj[0], h->S_adj[1], h->adj_mirror};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (h->h_ctrl) cudaFreeHost(h->h_ctrl);

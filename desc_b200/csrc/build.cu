@@ -108,7 +108,7 @@ __global__ void k_scan_nodes(const int* __restrict__ deg, int* __restrict__ rows
 __global__ void k_fill_adj(const int* __restrict__ ei, const int* __restrict__ ej, int64_t m,
                            const uint32_t* __restrict__ bm, const int* __restrict__ bmprefix,
                            int nwords, const int* __restrict__ rowstart, int* __restrict__ adj_nbr,
-                           int* __restrict__ adj_eid) {
+                           int* __restrict__ adj_eid, int* __restrict__ adj_mirror) {
     int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (e >= m) return;
     int i = ei[e], j = ej[e];
@@ -118,6 +118,7 @@ __global__ void k_fill_adj(const int* __restrict__ ei, const int* __restrict__ e
     adj_eid[pi] = (int)e;
     adj_nbr[pj] = i;
     adj_eid[pj] = (int)e;
+    adj_mirror[e] = pj;   // where the streamed PGD pass 1 stores the second copy of S[e] in adjacency order
 }
 
 // estart[v] = first edge whose smaller endpoint is >= v (edges sorted by (i,j)); estart[n] = m
@@ -183,6 +184,7 @@ int desc_graph_setup(desc_b200_handle* h, const double* d_Ind) {
     CUDA_TRY(cudaMalloc(&h->rowstart, (size_t)(n + 1) * sizeof(int)));
     CUDA_TRY(cudaMalloc(&h->adj_nbr, 2 * m * sizeof(int)));
     CUDA_TRY(cudaMalloc(&h->adj_eid, 2 * m * sizeof(int)));
+    CUDA_TRY(cudaMalloc(&h->adj_mirror, (m + 4) * sizeof(int)));   // +4: 16-byte widened bulk copies
     int* d_deg = nullptr;
     CUDA_TRY(cudaMalloc(&d_deg, (size_t)n * sizeof(int)));
     CUDA_TRY(cudaMemsetAsync(h->bm, 0, bmsz * sizeof(uint32_t), st));
@@ -193,7 +195,7 @@ int desc_graph_setup(desc_b200_handle* h, const double* d_Ind) {
     k_scan_nodes<<<1, 1024, 0, st>>>(d_deg, h->rowstart, n, h->d_err + 2);
     KERNEL_CHECK(h);
     k_fill_adj<<<gb, TB, 0, st>>>(h->ei, h->ej, m, h->bm, h->bmprefix, h->nwords, h->rowstart,
-                                  h->adj_nbr, h->adj_eid);
+                                  h->adj_nbr, h->adj_eid, h->adj_mirror);
     KERNEL_CHECK(h);
     CUDA_TRY(cudaMalloc(&h->estart, (size_t)(n + 1) * sizeof(int)));
     k_estart<<<(n + 1 + TB - 1) / TB, TB, 0, st>>>(h->ei, m, n, h->estart);

@@ -106,6 +106,7 @@ struct desc_b200_handle {
     int* rowstart = nullptr;    // n+1: CSR offsets of the symmetric adjacency
     int* adj_nbr = nullptr;     // 2m: neighbours, ascending within a row
     int* adj_eid = nullptr;     // 2m: edge id of (row, neighbour)
+    int* adj_mirror = nullptr;  // m+4: adjacency position of i in row j, for edge (i,j)
 
     // incidence -----------------------------------------------------------------------
     bool built = false, have_s0 = false, have_pgd = false;
@@ -143,8 +144,8 @@ struct desc_b200_handle {
     double* w[2] = {nullptr, nullptr};     // n_slots each (ping-pong)
     double* S[2] = {nullptr, nullptr};     // m each
     double* acc[2] = {nullptr, nullptr};   // 2m+2 each: partner sums via min/max endpoint, + [obj, change]
-    double* acc2[2] = {nullptr, nullptr};  // 2m each (streamed path, one GPU): the share of the pass over larger endpoints
-    double* S_adj = nullptr;                // 2m+4 (streamed path): S of the current state in adjacency order
+    double* P1 = nullptr;                   // 2m (streamed path, one GPU): pass 1's partner sums in adjacency order
+    double* S_adj[2] = {nullptr, nullptr};  // 2m+4 each (streamed path): S in adjacency order; [1] on one GPU only
     double* adam_m = nullptr;
     double* adam_v = nullptr;
     bool adam_valid = false;                // the Adam moments on this handle continue a rule with t > 0

@@ -39,7 +39,11 @@
 //    in-edges (u,v) with u < v) writes sjk = S_t[e_jk] for the next pass 1 and scatters "via j".  The
 //    scatters are read-modify-writes in warp-private tables (apices within one edge are distinct, one
 //    edge per warp instruction => no conflicts), flushed once per CTA.  No atomics: every partner-sum
-//    entry is owned by exactly one CTA per kernel, so the result is bit-reproducible.
+//    entry is owned by exactly one CTA per kernel, so the result is bit-reproducible.  On one GPU both
+//    passes keep their per-vertex data in adjacency order: pass 1 stores its partner sums into P1 and
+//    S_t into the next S_adj buffer (both copies of every edge), and pass 2 adds its sums to P1 and
+//    stores the finished (A, B) of every edge into acc_next.  Multi-GPU handles add both passes' sums
+//    into acc_next (one reduce-to-owners) and refill S_adj from the all-gathered S (k_pgd_s_adj).
 //  * blocked (k_pgd_block + k_pgd_scatter<false>): the same tables with direct loads and an L2 gather of
 //    S[e_jk].  Taken on single-GPU handles of sparse graphs (m < 100 n, where the streamed kernel's
 //    per-block prologue dominates), and when the streamed passes do not fit (slot lists longer than 256,
@@ -323,18 +327,26 @@ struct BlkArgs {
     int tstride;       // padded max degree (table stride)
     double* partial;   // 2 per CTA of k_pgd_block
     // streamed path only
-    const double* S_adj;   // S of the current state in adjacency order (k_pgd_s_adj)
-    const double* acc2_cur;  // partner sums of the pass over larger endpoints: read by the streamed kernel,
-    double* acc2_next;       //   written by the pass itself (both null on multi-GPU handles: it adds to acc_next)
+    const double* S_adj;   // S of the current state in adjacency order
+    // one GPU only (all three null on multi-GPU handles, whose pass 2 adds to acc_next and whose S_adj is refilled
+    // by k_pgd_s_adj after the all-gather):
+    double* P1;            // 2m: pass 1's partner sums in adjacency order; pass 2 adds its own and stores acc_next
+    double* S_adj_next;    // S of the state pass 1 builds, in adjacency order (pass 1 stores both copies of S[e])
+    const int* adj_mirror; // m: adjacency position of i in row j, for edge (i,j)
 };
 
 // shared tables: T_S[tstride] | T_acc[BLK_WARPS][tstride]
+// p1 non-null: the sums go to p1[rs + r] (adjacency order, plain stores); else added to the (edge, side) entries
 __device__ __forceinline__ void blk_flush(const BlkArgs& a, int v, int deg, int rs, const double* T_acc,
-                                          double* __restrict__ acc_out) {
+                                          double* __restrict__ acc_out, double* __restrict__ p1 = nullptr) {
     for (int r = threadIdx.x; r < deg; r += BLK_TB) {
         double x = 0.0;
 #pragma unroll
         for (int q = 0; q < BLK_WARPS; q++) x += T_acc[q * a.tstride + r];
+        if (p1) {
+            p1[rs + r] = x;
+            continue;
+        }
         const int e2 = a.adj_eid[rs + r];
         const int k = a.adj_nbr[rs + r];
         acc_out[2 * (int64_t)e2 + (v < k ? 0 : 1)] += x;   // owned by this CTA within this kernel
@@ -504,7 +516,8 @@ k_pgd_block(BlkArgs a) {
 }
 
 // Vertex-centric scatter of w (state being built) into acc_next.
-//   OUT = true : own edges (v,*) of the local range, ranks rk_i          (used for state 0 only)
+//   OUT = true : own edges (v,*) of the local range, ranks rk_i          (used for state 0 only; with P1 set,
+//                into P1 in adjacency order, the layout of the streamed pass 1, for pass 2 to finish)
 //   OUT = false: edges (u,v) with u < v, u in the local vertex range, ranks rk_j ("via j")
 // One warp handles one edge at a time (distinct ranks per instruction), four edges in flight.
 template <bool OUT>
@@ -527,7 +540,11 @@ k_pgd_scatter(BlkArgs a, const double* __restrict__ w) {
         lo = rs + (a.v0 > 0 ? desc_rank(a.bm, a.bmprefix, a.nwords, v, a.v0) : 0);
         hi = rs + desc_rank(a.bm, a.bmprefix, a.nwords, v, ub);
     }
-    if (hi <= lo) return;
+    if (hi <= lo) {
+        if (OUT && a.P1)   // P1 holds every row: no own edges, no "via i" sums
+            for (int r = threadIdx.x; r < deg; r += BLK_TB) a.P1[rs + r] = 0.0;
+        return;
+    }
     for (int r = threadIdx.x; r < deg; r += BLK_TB) {
 #pragma unroll
         for (int q = 0; q < BLK_WARPS; q++) T_acc[q * a.tstride + r] = 0.0;
@@ -574,7 +591,7 @@ k_pgd_scatter(BlkArgs a, const double* __restrict__ w) {
         }
     }
     __syncthreads();
-    blk_flush(a, v, deg, rs, T_acc, a.p.acc_next);
+    blk_flush(a, v, deg, rs, T_acc, a.p.acc_next, OUT ? a.P1 : nullptr);
 }
 
 // S in adjacency order, S_adj[p] = S[adj_eid[p]]: the table prologues of both streamed passes then read
@@ -642,7 +659,6 @@ static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, i
     sa.nstages = nst;
     sa.sjk = h->sjk;
     sa.S_adj = a.S_adj;
-    sa.acc2_cur = a.acc2_cur;
     const size_t smem = fixed + nst * stage;
     constexpr int NT = (NCW + NSW + 1) * 32;
     if (rule_kind == 0) {
@@ -748,7 +764,7 @@ static int launch_passb(desc_b200_handle* h, const BlkArgs& a, const double* w_t
 static int launch_s_adj(desc_b200_handle* h, const double* S) {
     const int64_t n2m = 2 * h->m;
     if (n2m == 0) return DESC_B200_OK;
-    k_pgd_s_adj<<<(unsigned)((n2m + 255) / 256), 256, 0, h->stream>>>(h->adj_eid, S, n2m, h->d_ctrl, h->S_adj);
+    k_pgd_s_adj<<<(unsigned)((n2m + 255) / 256), 256, 0, h->stream>>>(h->adj_eid, S, n2m, h->d_ctrl, h->S_adj[0]);
     KERNEL_CHECK(h);
     return DESC_B200_OK;
 }
@@ -932,8 +948,9 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
     ba.tstride = (h->maxdeg + 1 + 3) & ~3;   // >= maxdeg + 1: the last entry is a dummy slot for inactive lanes
     ba.partial = h->pgd_partial;
     ba.S_adj = nullptr;
-    ba.acc2_cur = nullptr;
-    ba.acc2_next = nullptr;
+    ba.P1 = nullptr;
+    ba.S_adj_next = nullptr;
+    ba.adj_mirror = h->adj_mirror;
     const size_t smem_blk = (size_t)(1 + BLK_WARPS) * ba.tstride * sizeof(double);
     const size_t smem_sc = (size_t)BLK_WARPS * ba.tstride * sizeof(double);
     const int launches0 = h->launches;
@@ -942,15 +959,17 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         stream = h->sjk != nullptr && launch_stream_any(h, ba, adam ? 1 : 0, true) == DESC_B200_OK &&
                  (size_t)(2 + 8) * ba.tstride * sizeof(double) <= 226 * 1024;
     }
+    // one GPU: pass 1 stores its partner sums in adjacency order (P1) and S_t in adjacency order (S_adj ping-pong);
+    // pass 2 adds its partner sums to P1 and stores the finished (A, B) of every edge.  Multi-GPU handles add both
+    // passes' sums into acc_next, reduce them to the owners, and refill one S_adj from the all-gathered S.
+    const bool use_p1 = stream && h->world == 1;
     if (stream) {
-        if (!h->S_adj) CUDA_TRY(cudaMalloc(&h->S_adj, (2 * m + 4) * sizeof(double)));   // +4: 16-byte widened bulk copies
-        ba.S_adj = h->S_adj;
-        // one GPU: the pass over larger endpoints stores its partner sums apart (no read-modify-write of acc)
-        if (h->world == 1)
-            for (int b = 0; b < 2; b++)
-                if (!h->acc2[b]) CUDA_TRY(cudaMalloc(&h->acc2[b], std::max<int64_t>(2 * m, 1) * sizeof(double)));
+        for (int b = 0; b < (use_p1 ? 2 : 1); b++)   // +4: 16-byte widened bulk copies
+            if (!h->S_adj[b]) CUDA_TRY(cudaMalloc(&h->S_adj[b], (2 * m + 4) * sizeof(double)));
+        if (use_p1 && !h->P1) CUDA_TRY(cudaMalloc(&h->P1, std::max<int64_t>(2 * m, 1) * sizeof(double)));
+        ba.S_adj = h->S_adj[0];
+        ba.P1 = use_p1 ? h->P1 : nullptr;
     }
-    const bool use_acc2 = stream && h->world == 1;
     const int G = h->max_ns <= 32 ? 8 : (h->max_ns <= 64 ? 16 : 32);
     const int aux_grid = DESC_SMS * 8;
 
@@ -979,10 +998,7 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
     }
     DESC_TRY(exchange_S(h, 0));
     if (stream) DESC_TRY(launch_s_adj(h, h->S[0]));   // needs every rank's S_0
-    if (stream && h->n_slots > 0) {
-        ba.acc2_next = use_acc2 ? h->acc2[0] : nullptr;
-        DESC_TRY(launch_passb(h, ba, h->w[0]));
-    }
+    if (stream && h->n_slots > 0) DESC_TRY(launch_passb(h, ba, h->w[0]));
     DESC_TRY(exchange_partner_sums(h, 0));
 
     // per-iteration kernel timing: events around the iteration kernels only
@@ -1018,18 +1034,22 @@ int desc_pgd_impl(desc_b200_handle* h, int iters, desc_b200_step_rule* rule, int
         const bool timed = t <= 512;
         if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1)], st));
         if (stream) {
-            // pass 1 (smaller endpoints): update; pass 2 (larger endpoints) needs all of S_t.  One S_adj serves
-            // pass 2 of iteration t and pass 1 of iteration t+1 (stream order).  It is no output: once the lagged
-            // stop flag is set every later kernel (the relayout too) returns, and the results are read from
-            // the ping-ponged S / w.
+            // pass 1 (smaller endpoints): update; pass 2 (larger endpoints) needs all of S_t.  S_t in adjacency
+            // order serves pass 2 of iteration t and pass 1 of iteration t+1 (stream order): on one GPU pass 1
+            // stores it into the other S_adj buffer, on multi-GPU handles k_pgd_s_adj refills the one buffer after
+            // the all-gather.  It is no output: once the lagged stop flag is set every later kernel returns, and
+            // the results are read from the ping-ponged S / w.
             ba.p = a;
-            ba.acc2_cur = use_acc2 ? h->acc2[cur] : nullptr;
-            ba.acc2_next = use_acc2 ? h->acc2[nxt] : nullptr;
+            ba.S_adj = h->S_adj[use_p1 ? cur : 0];
+            ba.S_adj_next = use_p1 ? h->S_adj[nxt] : nullptr;
             DESC_TRY(launch_stream_any(h, ba, adam ? 1 : 0));
             if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 1], st));
             DESC_TRY(exchange_S(h, nxt));
             if (timed) CUDA_TRY(cudaEventRecord(evs[5 * (t - 1) + 2], st));
-            DESC_TRY(launch_s_adj(h, h->S[nxt]));   // timed with pass 2
+            if (use_p1)
+                ba.S_adj = h->S_adj[nxt];
+            else
+                DESC_TRY(launch_s_adj(h, h->S[nxt]));   // timed with pass 2
             DESC_TRY(launch_passb(h, ba, h->w[nxt]));
             k_pgd_partials<<<1, PGD_PART_TB, 0, st>>>(h->pgd_partial, h->v_end - h->v_begin, h->d_ctrl, h->acc[nxt] + 2 * m);
             KERNEL_CHECK(h);

@@ -11,11 +11,13 @@
 // the (w, rank) loads of the next two batches of edges and the headers of the third in flight in
 // registers while it works on the current batch.
 // No atomics: every partner-sum entry (edge, side v) is owned by vertex v's CTA.
-// The S table is a contiguous read of S_adj (S in adjacency order, k_pgd_s_adj).  The partner sums
-// go to acc2_next with plain stores, every entry of the vertex's row in every launch (zeros when the
-// vertex has no local in-edges); the streamed kernel of the next iteration adds them to its own
-// (acc).  Multi-GPU handles (acc2_next null) add them to acc_next instead, so that one exchange
-// reduces the whole sum to the owners.
+// The S table is a contiguous read of S_adj (S in adjacency order).  On one GPU the flush finishes the
+// partner sums: it adds the table to pass 1's share of the same row, P1[rs + r], and stores the sum into
+// acc_next, every entry of the vertex's row in every launch (also when the vertex has no local
+// in-edges).  Positions r >= low (the upper neighbours) are the vertex's own edges estart[v] + r - low in
+// order, side A: contiguous stores.  Positions r < low are in-edges, side B: one adj_eid load and one
+// scattered store each.  Multi-GPU handles (P1 null) add the table to acc_next instead, so that one
+// exchange reduces the whole sum to the owners.
 #ifndef PB_U
 #define PB_U 4
 #endif
@@ -30,10 +32,35 @@
 __device__ __forceinline__ int64_t pb_acc_pos(const BlkArgs& a, int v, int rs, int r) {
     return 2 * (int64_t)a.adj_eid[rs + r] + (v < a.adj_nbr[rs + r] ? 0 : 1);
 }
-// a vertex without local in-edges: its row of acc2_next is zero in this launch
-__device__ __forceinline__ void pb_zero_row(const BlkArgs& a, int v, int rs, int deg) {
-    if (!a.acc2_next) return;
-    for (int r = threadIdx.x; r < deg; r += blockDim.x) a.acc2_next[pb_acc_pos(a, v, rs, r)] = 0.0;
+// One GPU: acc_next of v's row = P1 (pass 1's share) + the sum of the NQ tables T_acc (this pass's share, zero
+// when T_acc is null), by a CTA of NQ warps, KU entries per thread at a time so that the loads overlap
+template <int NQ, int KU>
+__device__ __forceinline__ void pb_finish_row(const BlkArgs& a, int v, int rs, int deg, const double* T_acc) {
+    const int eb = a.estart[v];
+    const int low = deg - (a.estart[v + 1] - eb);   // in-edges (u, v), u < v, come first in the row
+    constexpr int NT = NQ * 32;
+    for (int rb = threadIdx.x; rb < deg; rb += NT * KU) {
+        double p1[KU];
+        int e[KU];
+#pragma unroll
+        for (int k = 0; k < KU; k++) {
+            const int r = rb + k * NT;
+            p1[k] = r < deg ? a.P1[rs + r] : 0.0;
+            e[k] = r < low ? a.adj_eid[rs + r] : eb + r - low;
+        }
+#pragma unroll
+        for (int k = 0; k < KU; k++) {
+            const int r = rb + k * NT;
+            if (r < deg) {
+                double x = 0.0;
+                if (T_acc) {
+#pragma unroll
+                    for (int q = 0; q < NQ; q++) x += T_acc[q * a.tstride + r];
+                }
+                a.p.acc_next[2 * (int64_t)e[k] + (r < low ? 1 : 0)] = p1[k] + x;   // x1 + x2, as multi-GPU forms it
+            }
+        }
+    }
 }
 
 // PB_WARPS warps (= private tables) per CTA: 8 when a vertex has hundreds of local in-edges, fewer
@@ -53,21 +80,21 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
     const int v = (int)gridDim.x - 1 - (int)blockIdx.x;   // long in-edge lists first
     const int rs = a.rowstart[v];
     const int deg = a.rowstart[v + 1] - rs;
+    // (KU grows as the CTA shrinks: a 2-warp CTA - multi-GPU shards - still covers ~1280 entries per trip)
+    constexpr int KU = 40 / PB_WARPS;
     const int ub = min(a.v1, v);                           // neighbours u with v0 <= u < ub
     if (ub <= a.v0) {
-        pb_zero_row(a, v, rs, deg);
+        if (a.P1) pb_finish_row<PB_WARPS, KU>(a, v, rs, deg, nullptr);
         return;
     }
     const int lo = rs + (a.v0 > 0 ? desc_rank(a.bm, a.bmprefix, a.nwords, v, a.v0) : 0);
     const int hi = rs + desc_rank(a.bm, a.bmprefix, a.nwords, v, ub);
     if (hi <= lo) {
-        pb_zero_row(a, v, rs, deg);
+        if (a.P1) pb_finish_row<PB_WARPS, KU>(a, v, rs, deg, nullptr);
         return;
     }
     int2* shdr = reinterpret_cast<int2*>(T_acc + (size_t)PB_WARPS * a.tstride);   // headers of the in-edges [lo, hi)
     // table prologue, KU entries per thread at a time: all loads in flight together
-    // (KU grows as the CTA shrinks: a 2-warp CTA - multi-GPU shards - still covers ~1280 entries per trip)
-    constexpr int KU = 40 / PB_WARPS;
     for (int rb = threadIdx.x; rb < deg; rb += PB_TB * KU) {
         double sv[KU];
         int2 hv[KU];
@@ -181,9 +208,12 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
         base += 3 * stride;
     }
     __syncthreads();
-    // flush (every entry (edge, side v) is owned by this CTA within this kernel), KU entries per
-    // thread at a time so that the index loads (and, multi-GPU, the read-modify-writes) overlap
-    double* const out = a.acc2_next ? a.acc2_next : a.p.acc_next;
+    // flush (every entry (edge, side v) is owned by this CTA within this kernel)
+    if (a.P1) {
+        pb_finish_row<PB_WARPS, KU>(a, v, rs, deg, T_acc);
+        return;
+    }
+    // multi-GPU: KU entries per thread at a time so that the index loads and read-modify-writes overlap
     for (int rb = threadIdx.x; rb < deg; rb += PB_TB * KU) {
         int64_t pos[KU];
         double old[KU];
@@ -193,7 +223,7 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
             pos[k] = r < deg ? pb_acc_pos(a, v, rs, r) : -1;
         }
 #pragma unroll
-        for (int k = 0; k < KU; k++) old[k] = (!a.acc2_next && pos[k] >= 0) ? a.p.acc_next[pos[k]] : 0.0;
+        for (int k = 0; k < KU; k++) old[k] = pos[k] >= 0 ? a.p.acc_next[pos[k]] : 0.0;
 #pragma unroll
         for (int k = 0; k < KU; k++) {
             const int r = rb + k * PB_TB;
@@ -201,7 +231,7 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
                 double x = 0.0;
 #pragma unroll
                 for (int q = 0; q < PB_WARPS; q++) x += T_acc[q * a.tstride + r];
-                out[pos[k]] = a.acc2_next ? x : old[k] + x;
+                a.p.acc_next[pos[k]] = old[k] + x;
             }
         }
     }

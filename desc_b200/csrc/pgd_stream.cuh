@@ -9,8 +9,13 @@
 //     lists are contiguous) and per-edge arrays (rowptr, partner sums, S) into a ring of shared-
 //     memory stages; completion is signalled on an mbarrier (complete_tx::bytes).  L2 policy
 //     evict_first for the slot streams: they must not evict S.  Before the first tile it copies the
-//     vertex's S table, S_adj[rowstart[v] .. rowstart[v+1]) (S in adjacency order, k_pgd_s_adj),
-//     with one more bulk copy on its own mbarrier: no index-dependent gather in the prologue.
+//     vertex's S table, S_adj[rowstart[v] .. rowstart[v+1]) (S in adjacency order), with one more
+//     bulk copy on its own mbarrier: no index-dependent gather in the prologue.
+//   * One GPU: the compute warps store both adjacency-order copies of S_t[e] into the next S_adj
+//     buffer (the upper end of row i, contiguous, and adj_mirror[e] in row j, copied with the tile),
+//     and the flush stores the partner-sum table into P1 in adjacency order; pass 2 finishes the sums.
+//     Multi-GPU handles store the table into acc_next's (edge, side) entries and refill S_adj after
+//     the all-gather (k_pgd_s_adj).
 //   * COMPUTE warps: G lanes own one edge and keep EPL slots each in registers.  They read the
 //     stage, compute gradient / step / projection, write w_t in place into the stage, publish
 //     (slot offset, count) of their edges and arrive on the stage's `done` mbarrier.  There is NO
@@ -94,15 +99,17 @@ struct StreamArgs {
     int max_ns;       // longest slot list (size of the reciprocal table)
     const double* sjk;  // S[e_jk] per slot for the current state (pgd_passb.cuh)
     const double* S_adj;    // S_cur in adjacency order (2m + 4: 16-byte widened bulk copy)
-    const double* acc2_cur; // partner sums of the pass over larger endpoints (2m), null on multi-GPU handles
 };
 
 // shared-memory carve-up: barriers | edge headers[nstages][TE] | 1/c table | T_S[tstride+2] | T_acc[NSW] | stages.
 // One stage: w[tsc] f64 | S0[tsc] f64 | sjk[tsc] f64 | rk_i[tsc] u16 | rowptr[TE+2] i64 |
-//            acc_cur[2*TE] f64 | acc2_cur[2*TE] f64 | S_cur[TE+2] f64   (every offset a multiple of 16 bytes)
+//            acc_cur[2*TE] f64 | S_cur[TE+2] f64 | adj_mirror[st_mir_cap] i32   (every offset a multiple of 16 bytes)
 // The edge headers of a stage (st_hdr_bytes) sit apart from its ring slot, so only the stages in use take room.
+// adj_mirror is copied from a multiple of 4 edges: TE + 3 + 3 entries at most, rounded up to 4.
+__host__ __device__ __forceinline__ int st_mir_cap(int te) { return (te + 9) & ~3; }
 __host__ __device__ __forceinline__ size_t st_stage_bytes(int tsc, int te) {
-    return (size_t)tsc * (8 + 8 + 8 + 2) + (size_t)(te + 2) * 8 + (size_t)te * 32 + (size_t)(te + 2) * 8;
+    return (size_t)tsc * (8 + 8 + 8 + 2) + (size_t)(te + 2) * 8 + (size_t)te * 16 + (size_t)(te + 2) * 8 +
+           (size_t)st_mir_cap(te) * 4;
 }
 __host__ __device__ __forceinline__ size_t st_hdr_bytes(int te) { return (size_t)te * sizeof(int2); }
 __host__ __device__ __forceinline__ size_t st_rcp_bytes(int max_ns) { return ((size_t)(max_ns + 1) * 8 + 15) & ~(size_t)15; }
@@ -134,8 +141,8 @@ k_pgd_stream(StreamArgs sa) {
     const int tsc = sa.tsc;
     const size_t stage_bytes = st_stage_bytes(tsc, TE);
     const size_t off_d = (size_t)tsc * 8, off_sj = (size_t)tsc * 16, off_rk = (size_t)tsc * 24;
-    const size_t off_rp = (size_t)tsc * 26, off_acc = off_rp + (size_t)(TE + 2) * 8, off_acc2 = off_acc + (size_t)TE * 16;
-    const size_t off_so = off_acc2 + (size_t)TE * 16;
+    const size_t off_rp = (size_t)tsc * 26, off_acc = off_rp + (size_t)(TE + 2) * 8;
+    const size_t off_so = off_acc + (size_t)TE * 16, off_mi = off_so + (size_t)(TE + 2) * 8;
     const int NST = sa.nstages;
 
     const int v = a.v0 + blockIdx.x;
@@ -145,6 +152,10 @@ k_pgd_stream(StreamArgs sa) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (e_hi <= e_lo) {   // no own edges: nothing to update; its partner-sum entries start at zero
         for (int r = threadIdx.x; r < deg; r += NTHREADS) {
+            if (a.P1) {
+                a.P1[rs + r] = 0.0;
+                continue;
+            }
             const int e2 = a.adj_eid[rs + r];
             const int k = a.adj_nbr[rs + r];
             a.p.acc_next[2 * (int64_t)e2 + (v < k ? 0 : 1)] = 0.0;
@@ -208,16 +219,17 @@ k_pgd_stream(StreamArgs sa) {
                     const int e0a = e0 - eoff;
                     const int rp_cnt = (e1 + 1 - e0a + 1) & ~1;
                     const int so_cnt = (e1 - e0a + 1) & ~1;
+                    const int e0m = e0 & ~3;   // adj_mirror (4-byte entries): from a multiple of 4 edges
+                    const int mi_cnt = a.S_adj_next ? (e1 - e0m + 3) & ~3 : 0;
                     const int64_t base = sA & ~(int64_t)7;
                     const int64_t cnt = ((sB + 7) & ~(int64_t)7) - base;
                     unsigned char* st = stage0 + (size_t)s * stage_bytes;
                     mbar_wait(&empty[s], ph ^ 1u);
-                    mbar_expect_tx(&full[s], (uint32_t)(cnt * 26 + rp_cnt * 8 + (e1 - e0) * (sa.acc2_cur ? 32 : 16) + so_cnt * 8));
+                    mbar_expect_tx(&full[s], (uint32_t)(cnt * 26 + rp_cnt * 8 + (e1 - e0) * 16 + so_cnt * 8 + mi_cnt * 4));
                     bulk_g2s_plain(st + off_rp, a.p.rowptr + e0a, (uint32_t)(rp_cnt * 8), &full[s]);
                     bulk_g2s_plain(st + off_acc, a.p.acc_cur + 2 * (int64_t)e0, (uint32_t)((e1 - e0) * 16), &full[s]);
-                    if (sa.acc2_cur)
-                        bulk_g2s_plain(st + off_acc2, sa.acc2_cur + 2 * (int64_t)e0, (uint32_t)((e1 - e0) * 16), &full[s]);
                     bulk_g2s_plain(st + off_so, a.p.S_cur + e0a, (uint32_t)(so_cnt * 8), &full[s]);
+                    if (mi_cnt > 0) bulk_g2s_plain(st + off_mi, a.adj_mirror + e0m, (uint32_t)(mi_cnt * 4), &full[s]);
                     if (cnt > 0) {
                         bulk_g2s(st, a.p.w_cur + base, (uint32_t)(cnt * 8), &full[s], pol);
                         bulk_g2s(st + off_d, a.p.S0 + base, (uint32_t)(cnt * 8), &full[s], pol);
@@ -255,6 +267,7 @@ k_pgd_stream(StreamArgs sa) {
             const int g = (threadIdx.x & 31) / G;
             const int q = (threadIdx.x >> 5) * GPW + (GPW >= 4 ? 2 * (g % (GPW / 2)) + g / (GPW / 2) : g);
             const double nlr = -a.p.lr;
+            const int up = rs + deg - e_hi;   // S_adj position of own edge e: up + e (the upper end of the row)
             int s = 0;
             uint32_t ph = 0;
             unsigned char* st = stage0;
@@ -273,11 +286,6 @@ k_pgd_stream(StreamArgs sa) {
                     const double2 ab = reinterpret_cast<const double2*>(st + off_acc)[q];
                     A = ab.x;
                     B = ab.y;
-                    if (sa.acc2_cur) {   // x1 + x2: the sum the read-modify-write of the multi-GPU flush forms
-                        const double2 ab2 = reinterpret_cast<const double2*>(st + off_acc2)[q];
-                        A = ab.x + ab2.x;
-                        B = ab.y + ab2.y;
-                    }
                     Sold = (reinterpret_cast<const double*>(st + off_so) + eoff)[q];
                 }
                 const int nx = (ns - r + G - 1) / G;   // this lane owns slots x < nx  (G is a power of two)
@@ -373,6 +381,13 @@ k_pgd_stream(StreamArgs sa) {
                     if (ns > 0) {
                         a.p.S_next[e] = snew;
                         chgp += fabs(snew - Sold);
+                    }
+                    if (a.S_adj_next && e < e_hi) {
+                        // S_t in adjacency order, both copies: (i, j) in row i (contiguous: the own edges are
+                        // the upper end of the row) and (j, i) in row j.  An edge without slots keeps its S.
+                        const double sv = ns > 0 ? snew : Sold;
+                        a.S_adj_next[up + e] = sv;
+                        a.S_adj_next[(reinterpret_cast<const int*>(st + off_mi) + ((e - q) & 3))[q]] = sv;
                     }
                 }
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // w_t tile: generic writes -> bulk store
@@ -484,10 +499,18 @@ k_pgd_stream(StreamArgs sa) {
         }
     }
     __syncthreads();
-    // flush the private tables: every (edge, side) entry belongs to exactly one vertex block, and this
-    // kernel is the first writer of acc_next in an iteration => plain stores (the pass over larger
-    // endpoints stores its share into acc2_next, or adds it here on multi-GPU handles)
-    {
+    // flush the private tables: every (edge, side) entry belongs to exactly one vertex block.  One GPU: into
+    // P1 in adjacency order, contiguous (pass 2 adds its share and stores the finished sums into acc_next).
+    // Multi-GPU: this kernel is the first writer of acc_next in an iteration => plain stores (pass 2 adds
+    // its share to them).
+    if (a.P1) {
+        for (int r = threadIdx.x; r < deg; r += NTHREADS) {
+            double x = 0.0;
+#pragma unroll
+            for (int q = 0; q < ST_NSW; q++) x += T_acc[q * a.tstride + r];
+            a.P1[rs + r] = x;
+        }
+    } else {
         constexpr int KU = 4;
         for (int rb = threadIdx.x; rb < deg; rb += NTHREADS * KU) {
             int64_t pos[KU];
