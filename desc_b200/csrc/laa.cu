@@ -15,6 +15,7 @@
 #include "internal.cuh"
 
 #include <algorithm>
+#include <cstdlib>
 #include <cmath>
 
 namespace {
@@ -464,6 +465,10 @@ int desc_laa_impl(desc_b200_handle* h, const double* d_S, const double* d_Rinit,
     };
     const unsigned gm = (unsigned)((m + LAA_TB - 1) / LAA_TB), gn = (unsigned)((n + LAA_TB - 1) / LAA_TB);
     const unsigned gw = (unsigned)(((int64_t)n * 32 + LAA_TB - 1) / LAA_TB);
+    // CG needs at most n - 1 steps in exact arithmetic; 2n leaves room for rounding on slow-mixing graphs (rings
+    // need thousands of steps after the weights are truncated).  DESC_B200_LAA_CG_MAX overrides the cap (tests).
+    int cg_max = std::max(1000, 2 * n);
+    if (const char* o = getenv("DESC_B200_LAA_CG_MAX")) cg_max = std::max(1, atoi(o));
 
     k_laa_r2q<<<gn, LAA_TB, 0, st>>>(d_Rinit, n, 0, Q);
     KERNEL_CHECK(h);
@@ -495,7 +500,6 @@ int desc_laa_impl(desc_b200_handle* h, const double* d_S, const double* d_Rinit,
         CUDA_TRY(cudaMemcpyAsync(hs, sc, 16 * sizeof(double), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         const double bb[3] = {hs[12], hs[13], hs[14]};
-        const int cg_max = 1000;
         bool conv = (bb[0] == 0.0 && bb[1] == 0.0 && bb[2] == 0.0);
         for (int k = 1; k <= cg_max && !conv; k++) {
             k_laa_matvec<<<gw, LAA_TB, 0, st>>>(h->rowstart, h->adj_nbr, w2adj, P, n, AP);
@@ -520,6 +524,15 @@ int desc_laa_impl(desc_b200_handle* h, const double* d_S, const double* d_Rinit,
             }
         }
         CUDA_TRY(cudaGetLastError());
+        if (!conv) {   // an unconverged solve would move every node by a wrong step and still report success
+            double rel = 0.0;
+            for (int c = 0; c < 3; c++)
+                if (bb[c] > 0.0) rel = std::max(rel, std::sqrt(hs[9 + c] / bb[c]));
+            desc_set_error("LAA refinement: CG did not reach |r| <= 1e-13 |b| in %d iterations (relative residual %.3e) "
+                           "in IRLS iteration %d", cg_max, rel, it);
+            rc = DESC_B200_ERR_NOCONV;
+            break;
+        }
         // ---- node update, score
         k_laa_node_update<<<LAA_RED_BLOCKS, LAA_TB, 0, st>>>(n, X, Q, Wq, partial);
         KERNEL_CHECK(h);

@@ -547,11 +547,12 @@ def pgd(inc: Incidence, S0, iters, rule, patience=30, tol=1e-5, verbose=False, r
 # --------------------------------------------------------------------------------------
 
 
-def gcw(Ind, RijMat, S_vec, dense_limit=400, power=1.5):
+def gcw(Ind, RijMat, S_vec, dense_limit=400, power=1.5, return_eigs=False):
     """Top-3 eigenvectors ('la') of D^-1 (W o R), computed through the similar symmetric matrix
     D^-1/2 (W o R) D^-1/2 (SURVEY H4), unit 2-norm columns, sign rule GCW.m:28, SVD projection :30-36.
     ``power=1.5``: GCW.m:20;  ``power=1``: the weights of CEMP_GCW.m:141, ``1./(S+1e-8)`` (the rest of
-    CEMP_GCW.m:127-159 is GCW.m line for line)."""
+    CEMP_GCW.m:127-159 is GCW.m line for line).  ``return_eigs``: also return the largest eigenvalues of the
+    symmetric matrix in descending order (four with the dense solve, three with the sparse one)."""
     n, ei, ej = check_ind(Ind)
     R = to_internal(RijMat)
     S_vec = np.asarray(S_vec, dtype=np.float64).ravel()
@@ -570,6 +571,7 @@ def gcw(Ind, RijMat, S_vec, dense_limit=400, power=1.5):
         N[ej, :, ei, :] = blk.transpose(0, 2, 1)
         N = N.reshape(3 * n, 3 * n)
         lam, U = np.linalg.eigh(N)
+        lam = lam[::-1][:4]
         U = U[:, ::-1][:, :3]
     else:
         import scipy.sparse as sp
@@ -580,11 +582,13 @@ def gcw(Ind, RijMat, S_vec, dense_limit=400, power=1.5):
         Msp = Msp + Msp.T
         lam, U = eigsh(Msp, k=3, which="LA", tol=1e-14)
         U = U[:, np.argsort(-lam)]
+        lam = np.sort(lam)[::-1]
     V = U * np.repeat(isd, 3)[:, None]
     V = V / np.linalg.norm(V, axis=0, keepdims=True)
     if np.linalg.det(V[:3, :]) < 0:                              # GCW.m:28
         V[:, 0] = -V[:, 0]
-    return to_matlab(proj_so3(V.reshape(n, 3, 3)))               # GCW.m:30-36
+    R_est = to_matlab(proj_so3(V.reshape(n, 3, 3)))              # GCW.m:30-36
+    return (R_est, lam) if return_eigs else R_est
 
 
 # --------------------------------------------------------------------------------------
