@@ -689,7 +689,7 @@ template <int T>
 static int launch_fill_reg(desc_b200_handle* h, const FillArgs& fa) {
     const size_t smem = (size_t)8 * 32 * T * sizeof(int);
     CUDA_TRY(cudaFuncSetAttribute(k_fill_slots_reg<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int ctas = T <= 8 ? 8 : (T <= 16 ? 4 : 2);
+    const int ctas = T <= 8 ? 8 : 4;
     k_fill_slots_reg<T><<<DESC_SMS * ctas, 256, smem, h->stream>>>(fa);
     KERNEL_CHECK(h);
     return DESC_B200_OK;
@@ -740,19 +740,6 @@ __global__ void k_fill_explicit(FillArgs a, int* __restrict__ err) {
 // A4: reciprocal-slot flags.  Slot (ij;k): IKJ_appears <=> j is in the apex list of edge {i,k};
 // JKI_appears <=> i is in the apex list of edge {j,k}  (DESC.m:111-125).
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ bool apex_bsearch(const int* __restrict__ apex, int64_t lo, int64_t hi,
-                                             int v) {
-    const int64_t end = hi;
-    while (lo < hi) {
-        int64_t mid = (lo + hi) >> 1;
-        if (apex[mid] < v)
-            lo = mid + 1;
-        else
-            hi = mid;
-    }
-    return lo < end && apex[lo] == v;
-}
-
 __device__ __forceinline__ bool apex_lsearch(const int* __restrict__ apex, int64_t lo, int64_t hi,
                                              int v) {
     for (int64_t s = lo; s < hi; s++)
@@ -760,7 +747,7 @@ __device__ __forceinline__ bool apex_lsearch(const int* __restrict__ apex, int64
     return false;
 }
 
-template <bool SORTED>
+// explicit cycle lists (in any order): a linear search of the partner edges' apex lists
 __global__ void k_recip_flags(const int* __restrict__ ei, const int* __restrict__ ej,
                               const int64_t* __restrict__ rowptr, const int* __restrict__ apex,
                               uint32_t* __restrict__ pk_jk, uint32_t* __restrict__ pk_ki,
@@ -775,10 +762,8 @@ __global__ void k_recip_flags(const int* __restrict__ ei, const int* __restrict_
         for (int64_t s = r0 + lane; s < r1; s += 32) {
             uint32_t pki = pk_ki[s - slot_base], pjk = pk_jk[s - slot_base];
             int64_t eik = pki & PK_MASK, ejk = pjk & PK_MASK;
-            bool fa = SORTED ? apex_bsearch(apex, rowptr[eik], rowptr[eik + 1], j)
-                             : apex_lsearch(apex, rowptr[eik], rowptr[eik + 1], j);
-            bool fb = SORTED ? apex_bsearch(apex, rowptr[ejk], rowptr[ejk + 1], i)
-                             : apex_lsearch(apex, rowptr[ejk], rowptr[ejk + 1], i);
+            bool fa = apex_lsearch(apex, rowptr[eik], rowptr[eik + 1], j);
+            bool fb = apex_lsearch(apex, rowptr[ejk], rowptr[ejk + 1], i);
             pk_ki[s - slot_base] = (pki & ~PK_APP) | (fa ? PK_APP : 0u);
             pk_jk[s - slot_base] = (pjk & ~PK_APP) | (fb ? PK_APP : 0u);
             if (rk_i) {
@@ -791,7 +776,7 @@ __global__ void k_recip_flags(const int* __restrict__ ei, const int* __restrict_
 
 // Reciprocal-slot flags for the hash sampler (DESC.m:98-127): apex j is in the sampled list of edge
 // {i,k} iff (key(seed, e_ik, j), j) <= that edge's threshold pair: two table lookups per slot instead
-// of two binary searches in the partner edges' apex lists.
+// of two searches in the partner edges' apex lists.
 __global__ void k_recip_flags_thr(const int* __restrict__ ei, const int* __restrict__ ej,
                                   const int64_t* __restrict__ rowptr, uint32_t* __restrict__ pk_jk,
                                   uint32_t* __restrict__ pk_ki, uint16_t* __restrict__ rk_i,
@@ -1031,7 +1016,6 @@ int desc_build_incidence_impl(desc_b200_handle* h, int n_sample_req, uint64_t se
         CUDA_TRY(cudaMemcpyAsync(h->rowptr, cyc_ptr, (m + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
         k_ns_from_ptr<<<gb, TB, 0, st>>>(h->rowptr, m, d_ns);
         KERNEL_CHECK(h);
-        h->apex_sorted = false;
     } else {
         int ns;
         if (n_sample_req > 0)
@@ -1060,42 +1044,28 @@ int desc_build_incidence_impl(desc_b200_handle* h, int n_sample_req, uint64_t se
         DESC_TRY(desc_exclusive_scan_i64(h, d_ns, h->rowptr, m));
         CUDA_TRY(cudaMemcpyAsync(&h->m_cycle, h->rowptr + m, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
-        h->apex_sorted = true;
     }
     h->max_ns = std::min(h->n_sample, std::max(maxc, 1));
     if (explicit_lists) h->max_ns = h->n_sample;
     t_ns.release();
 
     // ---- shard: slot-balanced contiguous edge ranges
-    // shard of this rank.  DESC_B200_FAKE_SHARD="r/N" (profiling only, single GPU): take the edge / slot range rank r
-    // of N would own, with no exchanges -- the kernels then do one rank's work of an N-GPU solve (results are NOT a
-    // solution: the other ranks' contributions are missing) so that they can be profiled with ncu on one GPU.
-    int sw = h->world, sr = h->rank;
-    if (h->world == 1) {
-        if (const char* fs = getenv("DESC_B200_FAKE_SHARD")) {
-            int r = 0, N = 1;
-            if (sscanf(fs, "%d/%d", &r, &N) == 2 && N >= 1 && N <= 64 && r >= 0 && r < N) {
-                sr = r;
-                sw = N;
-            }
-        }
-    }
-    h->shard_edges.assign(sw + 1, 0);
+    h->shard_edges.assign(h->world + 1, 0);
     {
         int64_t* d_b = nullptr;
-        CUDA_TRY(cudaMalloc(&d_b, (sw + 1) * sizeof(int64_t)));
-        k_shard_bounds<<<1, 64, 0, st>>>(h->rowptr, m, h->m_cycle, sw, d_b);
+        CUDA_TRY(cudaMalloc(&d_b, (h->world + 1) * sizeof(int64_t)));
+        k_shard_bounds<<<1, 64, 0, st>>>(h->rowptr, m, h->m_cycle, h->world, d_b);
         KERNEL_CHECK(h);
-        CUDA_TRY(cudaMemcpyAsync(h->shard_edges.data(), d_b, (sw + 1) * sizeof(int64_t),
+        CUDA_TRY(cudaMemcpyAsync(h->shard_edges.data(), d_b, (h->world + 1) * sizeof(int64_t),
                                  cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         CUDA_TRY(cudaFree(d_b));
     }
     // align shard boundaries to vertex blocks (all edges with the same smaller endpoint stay together)
     {
-        std::vector<int> v_of(sw + 1, 0);
-        v_of[sw] = n;
-        for (int r = 1; r < sw; r++) {
+        std::vector<int> v_of(h->world + 1, 0);
+        v_of[h->world] = n;
+        for (int r = 1; r < h->world; r++) {
             if (h->shard_edges[r] >= m) {
                 v_of[r] = n;
                 h->shard_edges[r] = m;
@@ -1104,9 +1074,8 @@ int desc_build_incidence_impl(desc_b200_handle* h, int n_sample_req, uint64_t se
                 h->shard_edges[r] = h->h_estart[v_of[r]];
             }
         }
-        // cost-model boundaries (DESC_B200_SHARD=slots keeps the slot-balanced ones)
-        const char* sm = getenv("DESC_B200_SHARD");
-        if (sw > 1 && !(sm && strcmp(sm, "slots") == 0) && h->blocked_ok) {
+        // cost-model boundaries
+        if (h->world > 1 && h->blocked_ok) {
             DescTmp t_cs;
             CUDA_TRY(t_cs.alloc((size_t)(n + 1) * sizeof(int64_t)));
             k_vertex_slots<<<(n + 1 + 255) / 256, 256, 0, st>>>(h->rowptr, h->estart, n, t_cs.as<int64_t>());
@@ -1116,21 +1085,21 @@ int desc_build_incidence_impl(desc_b200_handle* h, int n_sample_req, uint64_t se
             CUDA_TRY(cudaMemcpyAsync(cs.data(), t_cs.p, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
             CUDA_TRY(cudaMemcpyAsync(ca.data(), h->rowstart, (size_t)(n + 1) * sizeof(int), cudaMemcpyDeviceToHost, st));
             CUDA_TRY(cudaStreamSynchronize(st));
-            cost_model_bounds(cs, ca, n, sw, v_of);
-            for (int r = 1; r < sw; r++) h->shard_edges[r] = h->h_estart[v_of[r]];
+            cost_model_bounds(cs, ca, n, h->world, v_of);
+            for (int r = 1; r < h->world; r++) h->shard_edges[r] = h->h_estart[v_of[r]];
         }
-        h->v_begin = v_of[sr];
-        h->v_end = v_of[sr + 1];
+        h->v_begin = v_of[h->rank];
+        h->v_end = v_of[h->rank + 1];
     }
-    h->e_begin = h->shard_edges[sr];
-    h->e_end = h->shard_edges[sr + 1];
-    h->shard_slots.assign(sw + 1, 0);
-    for (int r = 0; r <= sw; r++)
+    h->e_begin = h->shard_edges[h->rank];
+    h->e_end = h->shard_edges[h->rank + 1];
+    h->shard_slots.assign(h->world + 1, 0);
+    for (int r = 0; r <= h->world; r++)
         CUDA_TRY(cudaMemcpyAsync(&h->shard_slots[r], h->rowptr + h->shard_edges[r], sizeof(int64_t),
                                  cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    h->slot_base = h->shard_slots[sr];
-    h->n_slots = h->shard_slots[sr + 1] - h->slot_base;
+    h->slot_base = h->shard_slots[h->rank];
+    h->n_slots = h->shard_slots[h->rank + 1] - h->slot_base;
 
     // + 16: the streamed PGD kernel widens its bulk copies to 16-byte boundaries (pgd_stream.cuh)
     const size_t ns_alloc = (size_t)std::max<int64_t>(h->n_slots, 1) + 16;
@@ -1167,10 +1136,6 @@ int desc_build_incidence_impl(desc_b200_handle* h, int n_sample_req, uint64_t se
     fa.rk_j = h->rk_j;
     fa.e0 = h->e_begin;
     fa.e1 = h->e_end;
-    if (sw != h->world) {   // profiling shard: no all-gather will deliver the other edges' lists / thresholds
-        fa.e0 = 0;
-        fa.e1 = m;
-    }
     fa.l0 = h->e_begin;
     fa.l1 = h->e_end;
     fa.slot_base = h->slot_base;
@@ -1212,19 +1177,15 @@ int desc_build_incidence_impl(desc_b200_handle* h, int n_sample_req, uint64_t se
             }
             fa.thr_key = h->thr_key;
             fa.thr_k = h->thr_k;
-            // register-resident selection for co-degrees up to 1024 (DESC_B200_FILL=generic forces the other kernel)
-            const char* fm = getenv("DESC_B200_FILL");
-            const bool generic = fm && strcmp(fm, "generic") == 0;
-            if (!generic && maxc <= 128) {
+            // register-resident selection for co-degrees up to 512.  Above, the shared-memory kernel: 32 candidate
+            // registers per lane needed 242 registers per thread and took 43 ms against its 11.5 ms at cfg 3
+            // (co-degrees ~500, profiles/README.md round 2)
+            if (maxc <= 128) {
                 DESC_TRY(launch_fill_reg<4>(h, fa));
-            } else if (!generic && maxc <= 256) {
+            } else if (maxc <= 256) {
                 DESC_TRY(launch_fill_reg<8>(h, fa));
-            } else if (!generic && maxc <= 512) {
+            } else if (maxc <= 512) {
                 DESC_TRY(launch_fill_reg<16>(h, fa));
-            } else if (!generic && maxc <= 1024 && fm && strcmp(fm, "reg32") == 0) {
-                // 32 candidate registers per lane need 242 registers per thread: measured 43 ms against the 11.5 ms
-                // of the shared-memory kernel at cfg 3 (co-degrees ~500), so this shape is opt-in only
-                DESC_TRY(launch_fill_reg<32>(h, fa));
             } else {
                 k_fill_slots<<<DESC_SMS * ctas_per_sm, wpb * 32, smem, st>>>(fa);
                 KERNEL_CHECK(h);
@@ -1237,12 +1198,10 @@ int desc_build_incidence_impl(desc_b200_handle* h, int n_sample_req, uint64_t se
         if (!explicit_lists) {
             k_recip_flags_thr<<<warp_grid, 256, 0, st>>>(h->ei, h->ej, h->rowptr, h->pk_jk, h->pk_ki, h->rk_i, h->rk_j,
                                                          h->thr_key, h->thr_k, seed, h->e_begin, h->e_end, h->slot_base);
-        } else if (h->apex_sorted)
-            k_recip_flags<true><<<warp_grid, 256, 0, st>>>(h->ei, h->ej, h->rowptr, h->apex, h->pk_jk, h->pk_ki,
-                                                          h->rk_i, h->rk_j, h->e_begin, h->e_end, h->slot_base);
-        else
-            k_recip_flags<false><<<warp_grid, 256, 0, st>>>(h->ei, h->ej, h->rowptr, h->apex, h->pk_jk, h->pk_ki,
-                                                           h->rk_i, h->rk_j, h->e_begin, h->e_end, h->slot_base);
+        } else {
+            k_recip_flags<<<warp_grid, 256, 0, st>>>(h->ei, h->ej, h->rowptr, h->apex, h->pk_jk, h->pk_ki, h->rk_i,
+                                                     h->rk_j, h->e_begin, h->e_end, h->slot_base);
+        }
         KERNEL_CHECK(h);
     }
     h->built = true;

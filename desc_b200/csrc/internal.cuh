@@ -110,7 +110,6 @@ struct desc_b200_handle {
 
     // incidence -----------------------------------------------------------------------
     bool built = false, have_s0 = false, have_pgd = false;
-    bool apex_sorted = true;
     int* codeg = nullptr;       // m
     uint64_t* thr_key = nullptr;  // m: sampler threshold of every edge = largest selected (key, apex) pair;
     int* thr_k = nullptr;         //    membership of an apex in an edge's sampled list is then one comparison

@@ -637,7 +637,7 @@ k_pgd_partials(const double* __restrict__ partial, int nblocks, const int* __res
 #include "pgd_passb.cuh"
 
 template <int G, int EPL, int NCW, int NSW>
-static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, int want_ctas, bool dry) {
+static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, bool dry) {
     const int nv = a.v1 - a.v0;
     if (nv <= 0) return DESC_B200_OK;
     constexpr int TE = NCW * 32 / G;
@@ -646,10 +646,10 @@ static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, i
     sa.max_ns = h->max_ns;
     sa.tsc = (TE * h->max_ns + G * EPL + 16 + 7) & ~7;
     const size_t fixed = st_fixed_bytes(a.tstride, h->max_ns, NSW), stage = st_stage_bytes(sa.tsc, TE) + st_hdr_bytes(TE);
-    // several CTAs per SM: one CTA's table prologue / flush overlaps the others' streaming.
+    // up to four CTAs per SM: one CTA's table prologue / flush overlaps the others' streaming.
     // 228 KB of shared memory per SM, 1 KB reserved per CTA.
     int nst = 0;
-    for (int ctas = want_ctas; ctas >= 1 && !nst; ctas--) {
+    for (int ctas = 4; ctas >= 1 && !nst; ctas--) {
         const size_t budget = (size_t)(228 * 1024) / ctas - 1024 - 256;
         for (int c = ST_MAXSTAGES; c >= 2 && !nst; c--)
             if (fixed + c * stage <= budget) nst = c;
@@ -672,34 +672,17 @@ static int launch_stream(desc_b200_handle* h, const BlkArgs& a, int rule_kind, i
     return DESC_B200_OK;
 }
 
-// slots-per-lane variants of one (compute warps, scatter warps) shape; lanes per edge follow max_ns
-template <int EPL, int NCW, int NSW>
-static int launch_stream_ns(desc_b200_handle* h, const BlkArgs& a, int rule_kind, int ctas, bool dry) {
-    const int ns = h->max_ns;
-    if (ns <= 32) return launch_stream<32 / EPL, EPL, NCW, NSW>(h, a, rule_kind, ctas, dry);
-    if (ns <= 64) return launch_stream<64 / EPL, EPL, NCW, NSW>(h, a, rule_kind, ctas, dry);
-    if (ns <= 128) return launch_stream<128 / EPL, EPL, NCW, NSW>(h, a, rule_kind, ctas, dry);
-    if (EPL >= 8 && ns <= 256) return launch_stream<(EPL >= 8 ? 256 / EPL : 32), EPL, NCW, NSW>(h, a, rule_kind, ctas, dry);
-    return DESC_B200_ERR_LIMIT;
-}
-
 // DESC_B200_ERR_LIMIT = this graph does not fit the streamed kernel (use the blocked one).
-// DESC_B200_ST="<slots per lane>,<compute warps>,<scatter warps>,<CTAs per SM>" picks another
-// compiled launch shape (experiments).
+// Launch shape: 8 slots per lane, 16-edge tiles of 2 compute + 2 scatter warps, up to four CTAs per SM -- the best of
+// the shapes measured at cfg 4 (profiles/README.md): smaller CTAs overlap each other's per-vertex prologue / drain
+// (round 2: 1.29 -> 1.24 ms).  Lanes per edge follow max_ns.
 static int launch_stream_any(desc_b200_handle* h, const BlkArgs& a, int rule_kind, bool dry = false) {
-    // best of the shapes measured at cfg 4 (profiles/README.md): 16-edge tiles, 2 compute + 2 scatter warps and four
-    // CTAs per SM -- smaller CTAs overlap each other's per-vertex prologue / drain (round 2: 1.29 -> 1.24 ms)
-    int epl = 8, ncw = 2, nsw = 2, ctas = 4;
-    if (const char* o = getenv("DESC_B200_ST")) sscanf(o, "%d,%d,%d,%d", &epl, &ncw, &nsw, &ctas);
-#define ST_CASE(E, C, S) \
-    if (epl == E && ncw == C && nsw == S) return launch_stream_ns<E, C, S>(h, a, rule_kind, ctas, dry);
-    ST_CASE(8, 4, 4)
-    ST_CASE(8, 4, 2)
-    ST_CASE(4, 8, 2)
-    ST_CASE(8, 2, 2)   // 16-edge tiles, 5 warps: three or four CTAs per SM (per-CTA prologue / drain overlap)
-#undef ST_CASE
-    desc_set_error("DESC_B200_ST=%d,%d,%d,%d is not a compiled launch shape", epl, ncw, nsw, ctas);
-    return DESC_B200_ERR_ARG;
+    const int ns = h->max_ns;
+    if (ns <= 32) return launch_stream<4, 8, 2, 2>(h, a, rule_kind, dry);
+    if (ns <= 64) return launch_stream<8, 8, 2, 2>(h, a, rule_kind, dry);
+    if (ns <= 128) return launch_stream<16, 8, 2, 2>(h, a, rule_kind, dry);
+    if (ns <= 256) return launch_stream<32, 8, 2, 2>(h, a, rule_kind, dry);
+    return DESC_B200_ERR_LIMIT;
 }
 
 template <int G, int EPL>
@@ -740,22 +723,18 @@ static int launch_scatter(desc_b200_handle* h, const BlkArgs& a, const double* w
 
 // pass over larger endpoints of the streamed path: sjk <- S_t[e_jk], partner sums "via j" of w_t
 static int launch_passb(desc_b200_handle* h, const BlkArgs& a, const double* w_t) {
-    // warps per CTA by the mean number of local in-edges per vertex (batches of PB_U edges per warp)
+    // warps per CTA by the mean number of local in-edges per vertex (batches of PB_U edges per warp).  Fewer than 4
+    // do not pay: measured on one rank's share of an 8-GPU solve, 4 warps beat 2 there (0.438 against 0.476 ms,
+    // profiles/README.md round 2)
     const double per_cta = (double)(h->e_end - h->e_begin) / std::max(h->n, 1);
-    // (2-warp CTAs were used for the small per-vertex work of 4-8 GPU shards; measured on one rank's share of an
-    // 8-GPU solve, 4 warps are faster there too: 0.476 -> 0.438 ms, profiles/README.md round 2)
-    int nw = per_cta >= 256 ? 8 : 4;
-    if (const char* o = getenv("DESC_B200_PB_WARPS")) {
-        if (atoi(o) > 0) nw = atoi(o);
-    }
-    nw = nw >= 8 ? 8 : (nw >= 4 ? 4 : 2);
+    const int nw = per_cta >= 256 ? 8 : 4;
     const size_t smem = (size_t)(2 + nw) * a.tstride * sizeof(double);   // T_S, nw private tables, header tile
 #define PB_LAUNCH(NW)                                                                                              \
     {                                                                                                              \
         CUDA_TRY(cudaFuncSetAttribute(k_pgd_passb<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));       \
         k_pgd_passb<NW><<<h->n, NW * 32, smem, h->stream>>>(a, w_t, h->jhdr, h->sjk, (h->max_ns + 31) / 32);           \
     }
-    if (nw >= 8) PB_LAUNCH(8) else if (nw >= 4) PB_LAUNCH(4) else PB_LAUNCH(2)
+    if (nw == 8) PB_LAUNCH(8) else PB_LAUNCH(4)
 #undef PB_LAUNCH
     KERNEL_CHECK(h);
     return DESC_B200_OK;

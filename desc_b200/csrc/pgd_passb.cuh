@@ -24,9 +24,6 @@
 #ifndef PB_PF
 #define PB_PF 6                         // L2 prefetch distance in batches
 #endif
-#ifndef PB_DEPTH
-#define PB_DEPTH 2                      // batches of (w, rank) loads in flight ahead of the current one
-#endif
 
 // partner-sum entry (edge, side v) of adjacency position rs + r of vertex v
 __device__ __forceinline__ int64_t pb_acc_pos(const BlkArgs& a, int v, int rs, int r) {
@@ -63,9 +60,9 @@ __device__ __forceinline__ void pb_finish_row(const BlkArgs& a, int v, int rs, i
     }
 }
 
-// PB_WARPS warps (= private tables) per CTA: 8 when a vertex has hundreds of local in-edges, fewer
-// (smaller CTAs, more of them per SM) when sharding over GPUs leaves each CTA little work, so that
-// the O(degree) table prologue / flush of one CTA overlaps the others'.
+// PB_WARPS warps (= private tables) per CTA: 8 when a vertex has hundreds of local in-edges, else 4
+// (smaller CTAs, more of them per SM), so that the O(degree) table prologue / flush of one CTA
+// overlaps the others'.
 template <int PB_WARPS>
 __global__ void __launch_bounds__(PB_WARPS * 32)
 k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jhdr, double* __restrict__ sjk,
@@ -80,7 +77,7 @@ k_pgd_passb(BlkArgs a, const double* __restrict__ w, const int2* __restrict__ jh
     const int v = (int)gridDim.x - 1 - (int)blockIdx.x;   // long in-edge lists first
     const int rs = a.rowstart[v];
     const int deg = a.rowstart[v + 1] - rs;
-    // (KU grows as the CTA shrinks: a 2-warp CTA - multi-GPU shards - still covers ~1280 entries per trip)
+    // (KU grows as the CTA shrinks: both shapes cover 1280 entries per trip)
     constexpr int KU = 40 / PB_WARPS;
     const int ub = min(a.v1, v);                           // neighbours u with v0 <= u < ub
     if (ub <= a.v0) {

@@ -402,6 +402,7 @@ def test_streamed_path_slot_list_lengths_and_rules(monkeypatch, ns, rule):
         rc, ro = desc_b200.HybridGradient(0.002, 0.9, 0.999, 25), O.HybridGradient(0.002, 0.9, 0.999, 25)
     c = run_cuda(mo["Ind"], mo["RijMat"], rc, 20, n_sample=ns, seed=4, gcw=False)
     assert c["timings"]["pgd_pass2_ms"] > 0.0                 # the two-pass streamed path ran
+    assert c["info"]["max_slots_per_edge"] > (32 if ns > 32 else 0)
     o = run_oracle(mo["Ind"], mo["RijMat"], ro, 20, n_sample=(None if ns == 0 else ns), seed=4, gcw=False)
     assert_incidence_equal(c, o["inc"])
     assert_solution_close(c, o)
@@ -472,20 +473,6 @@ def _cached_case(n, p, rng, lr, iters, ns, seed):
                        seed=seed, gcw=False)
         _ORACLE_CACHE[key] = (mo, o)
     return _ORACLE_CACHE[key]
-
-
-@pytest.mark.parametrize("shape", ["8,2,2,4", "8,4,4,2", "8,4,2,2", "4,8,2,2"])
-@pytest.mark.parametrize("ns", [0, 45, 100])
-def test_streamed_path_launch_shapes_and_slot_list_lengths(monkeypatch, shape, ns):
-    """every compiled (slots per lane, compute warps, scatter warps) shape of the TMA-streamed kernel, with
-    slot lists of <=32, <=64 and <=128 entries (4..16 or 8..32 lanes per edge), against the oracle"""
-    monkeypatch.setenv("DESC_B200_PGD_PATH", "stream")
-    monkeypatch.setenv("DESC_B200_ST", shape)
-    mo, o = _cached_case(240, 0.65, 34, 0.05, 20, ns, 4)
-    c = run_cuda(mo["Ind"], mo["RijMat"], desc_b200.ConstantStepSize(0.05), 20, n_sample=ns, seed=4, gcw=False)
-    assert c["info"]["max_slots_per_edge"] > (0 if ns == 0 else 32)
-    assert_incidence_equal(c, o["inc"])
-    assert_solution_close(c, o)
 
 
 @pytest.mark.parametrize("path", ["stream"])
